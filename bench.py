@@ -9,6 +9,7 @@ config 5 (16384^2, 256x256 window, sharded by tile row with NCCL halo rows).
 
   python bench.py --gpus N --steps K --warmup W          our arm (torchrun for N > 1)
   python bench.py --impl reference ...                   the reference algorithm on the host cores (rank 0 only)
+  python bench.py --gpus 1 ... --dump-outputs DIR        also write the headline disparity of the last timed step to DIR
 
 N > 1: the image is sharded into contiguous output-row bands, one per rank (strong scaling).  Inputs are row-sharded too:
 every step each rank receives the halo rows it needs (kernel-1 rows of the left raster, kernel-1 + search-1 rows of the
@@ -28,6 +29,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 COSTS = {"abs": 0, "sq": 1, "ncc": 2}
 # measured on this pool's B200 (tools/microbench.cu, profiles/microbench_r01.txt): 3.9 warp-instructions / clk / SM
@@ -51,7 +53,29 @@ def parse():
     ap.add_argument("--cfg5-size", type=int, default=0, help="run config 5 at this raster size on any N > 1 (default: 16384 at N = 8 only)")
     ap.add_argument("--cpu-tile", type=int, default=0, help="output tile per CPU thread of the reference arm (0 = the largest of "
                     "1024 / 512 / 256 / 128 whose step stays near 12 s; BASELINE.md asks for 1024^2 tiles)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the headline disparity of the last timed step as float32 .npy "
+                    "files under DIR (a fixed sample of rows when the whole raster is larger than DUMP_BYTES); --gpus 1 only")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.gpus != 1 or a.impl != "ours"):
+        ap.error("--dump-outputs needs --gpus 1 and --impl ours")
+    return a
+
+
+DUMP_BYTES = 48 << 20          # float32 disparity rows written by --dump-outputs (the row index adds a few KB)
+
+
+def dump_outputs(d, disp):
+    """disparity.npy: float32 (n, W, 3) {dx, dy, valid} rows of the (H, W, 3) int32 result; disparity_rows.npy: float64 (n,)
+    the row of each.  All rows when they fit in DUMP_BYTES, else a sorted sample drawn with a fixed seed, so that two
+    builds run with the same arguments write the same rows."""
+    H, W = disp.shape[:2]
+    n = min(H, max(1, DUMP_BYTES // (W * 3 * 4)))
+    rows = np.arange(H) if n == H else np.sort(np.random.default_rng(0).choice(H, n, replace=False))
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "disparity.npy"), disp[rows].astype(np.float32))
+    np.save(os.path.join(d, "disparity_rows.npy"), rows.astype(np.float64))
 
 
 def workload_name(a):
@@ -673,6 +697,8 @@ def run_ours(a):
     e2e = S * S * a.steps / (te * 1e-3) / 1e6
     out_np = out.cpu().numpy()
     same = bool(np.array_equal(hout_np, out_np))         # the e2e result must equal the device-resident result
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, out_np)
     # ---- sampled-tile parity of this run against the oracle (rank 0's band) ----
     parity = None
     if rank == 0:

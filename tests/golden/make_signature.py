@@ -1,6 +1,8 @@
 """Extract the parameter lists of PyramidCorrelationView's constructor and of pyramid_correlate() from the reference header
 (Stereo/CorrelationView.h:48-69, :195-218) into tests/golden/pyramid_correlate_signature.json -- the fixture
-tests/test_cpp_shim.py compares the shim with on boxes where /root/reference does not exist."""
+tests/test_cpp_shim.py compares the shim with.
+
+  python tests/golden/make_signature.py <Vision Workbench source tree>/src/vw/Stereo/CorrelationView.h"""
 import json
 import os
 import re
@@ -51,7 +53,6 @@ def extract(header_text):
 
 
 if __name__ == "__main__":
-    ref = sys.argv[1] if len(sys.argv) > 1 else "/root/reference/src/vw/Stereo/CorrelationView.h"
-    sig = extract(open(ref).read())
+    sig = extract(open(sys.argv[1]).read())
     json.dump(sig, open(os.path.join(HERE, "pyramid_correlate_signature.json"), "w"), indent=1)
     print(len(sig["constructor"]), len(sig["factory"]))

@@ -1,12 +1,12 @@
 """SemiGlobalMatcher core of the oracle (oracle/vw_sgm_oracle.c; SURVEY section 8 row a10): pinned by the reference's own
 known-answer test (Stereo/tests/TestSGM.cxx:27-75: constant offset (2,1), search [-4,4]^2, census 3x3, > 99 % correct)
--- on the reference's fixture images when they are present, and on a synthetic equivalent that is always run."""
+-- on a stored crop of the reference's fixture images, and on a synthetic equivalent."""
 import os
 
 import numpy as np
 import pytest
 
-REF_TESTS = "/root/reference/src/vw/Stereo/tests"
+SGM_FIXTURE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "sgm_fixture.npz")
 
 
 def _constant_offset_pair(seed, W=180, H=150, off=(2, 1), smin=(-4, -4), ssize=(9, 9)):
@@ -50,18 +50,14 @@ def test_sgm_rejects_unsupported_kernel(oracle):
         oracle.sgm_calc_disparity(left, right, (8, 8), 11)      # NoImplErr in the reference (SGM.cc:1885-1888)
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF_TESTS, "left.tif")), reason="reference fixtures not present")
 def test_sgm_reference_fixture_kat(oracle):
-    cv2 = pytest.importorskip("cv2")
-    L = cv2.imread(os.path.join(REF_TESTS, "left.tif"), cv2.IMREAD_UNCHANGED).astype(np.float32)
-    R = cv2.imread(os.path.join(REF_TESTS, "left_const_offset.tif"), cv2.IMREAD_UNCHANGED).astype(np.float32)
-    # TestSGM.cxx uses leftRoi (0,0,400,400), whose right ROI starts at (-4,-4); an interior ROI avoids reading outside the file
-    x0, y0, w, h = 8, 8, 380, 380
-    left = L[y0:y0 + h, x0:x0 + w]
-    right = R[y0 - 4:y0 - 4 + h + 9, x0 - 4:x0 - 4 + w + 9]
+    # TestSGM.cxx uses leftRoi (0,0,400,400), whose right ROI starts at (-4,-4); the stored interior ROI of its images
+    # (tests/golden/make_sgm_fixture.py) avoids reading outside the file
+    g = np.load(SGM_FIXTURE)
+    left, right = g["left"].astype(np.float32), g["right"].astype(np.float32)
     d = oracle.sgm_calc_disparity(left, right, (8, 8), 3)
-    dd = d[..., :2] + np.array([-4, -4])
-    assert ((dd[..., 0] == 2) & (dd[..., 1] == 1)).mean() > 0.99
+    dd = d[..., :2] + g["search_min"]
+    assert ((dd[..., 0] == g["offset"][0]) & (dd[..., 1] == g["offset"][1])).mean() > 0.99
 
 
 def test_sgm_per_pixel_boxes_reduce_to_the_constant_case(oracle):
