@@ -125,6 +125,44 @@ int vwb200_parabola_subpixel(const float* disparity, int cols, int rows, const f
                              float* dest, ptrdiff_t dest_pitch, int on_device, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * vw::stereo::PyramidSubpixelView::rasterize(dest, bbox) (src/vw/Stereo/SubpixelView.h:42-150,
+ * .cc:33-224): iterative sub-pixel refinement of a PixelMask<Vector2f> disparity over an image pyramid
+ * of max_pyramid_levels levels (< 0 is clamped to 0).  Arguments as vwb200_parabola_subpixel, plus the
+ * algorithm (PyramidSubpixelView_Algorithm).  dest: (x1-x0) x (y1-y0) triples, pitch in pixels.
+ * Results are bit-identical to the sequential reference order (DESIGN.md section K6).
+ * Odd kernel >= 3 and a bbox inside the image, else VWB200_EARG; SUBPIXEL_PHASE or an unknown
+ * algorithm -> VWB200_ENOIMPL.  A disparity value in the bbox that is NaN, infinite or of magnitude >= 2^24 -> VWB200_EARG.
+ * The call synchronises the stream (the disparity range is read back, and one flag per validity-fixpoint round).
+ * ------------------------------------------------------------------------------------------- */
+#define VWB200_SUBPIXEL_LUCAS_KANADE 0
+#define VWB200_SUBPIXEL_FAST_AFFINE  1
+#define VWB200_SUBPIXEL_BAYES_EM     2
+#define VWB200_SUBPIXEL_PHASE        3
+int vwb200_pyramid_subpixel(const float* disparity, int cols, int rows, const float* left, ptrdiff_t lpitch,
+                            const float* right, int rcols, int rrows, ptrdiff_t rpitch, int kx, int ky,
+                            int prefilter_mode, float prefilter_width, int x0, int y0, int x1, int y1,
+                            float* dest, ptrdiff_t dest_pitch, int on_device, void* stream,
+                            int max_pyramid_levels, int algorithm);
+/* One level function, in place: subpixel_optimized_LK_2d / subpixel_optimized_affine_2d /
+ * subpixel_optimized_affine_2d_EM (Stereo/Correlate.cc:500-1391, Correlate.h:63-104).  disparity: cols x rows
+ * triples (pitch in pixels), left: cols x rows, right: rcols x rrows.  roi = [x0,x1) x [y0,y1); the scan
+ * covers the roi grown by one pixel, clipped to the kernel's reach of the image. */
+int vwb200_subpixel_refine(int algorithm, float* disparity, int cols, int rows, ptrdiff_t dpitch,
+                           const float* left, ptrdiff_t lpitch, const float* right, int rcols, int rrows, ptrdiff_t rpitch,
+                           int kx, int ky, int x0, int y0, int x1, int y1, int do_h, int do_v, int on_device, void* stream);
+/* Counters of the calling thread's last vwb200_pyramid_subpixel / vwb200_subpixel_refine call.
+ * SIMT efficiency = window_evaluations / lane_slots. */
+typedef struct {
+  long long levels;               /* level-function runs */
+  long long fixpoint_rounds;      /* validity-fixpoint rounds summed over the levels */
+  long long pixels;               /* pixels in the scan regions */
+  long long pixels_reevaluated;   /* evaluations after round 0 */
+  long long window_evaluations;   /* window-pixel evaluations (passes x kx x ky) */
+  long long lane_slots;           /* sum over warps of 32 x the largest per-lane evaluation count */
+} vwb200_subpixel_stats;
+int vwb200_last_subpixel_stats(vwb200_subpixel_stats* out);
+
+/* ---------------------------------------------------------------------------------------------
  * vw::stereo::calc_disparity_sgm (src/vw/Stereo/SGM.cc:167-230, SGM.h:361-376) ->
  * SemiGlobalMatcher::semi_global_matching_func (:2387-2448): u8_convert, (ternary) census costs for kernel 3/5/7/9,
  * per-pixel search boxes, SGM or MGM accumulation along 8 directions, integer winner with the reference's tie

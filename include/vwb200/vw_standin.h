@@ -176,5 +176,7 @@ struct SemiGlobalMatcher {                                                      
 enum CostFunctionType { ABSOLUTE_DIFFERENCE, SQUARED_DIFFERENCE, CROSS_CORRELATION, CENSUS_TRANSFORM, TERNARY_CENSUS_TRANSFORM };  // Stereo/CostFunctions.h:143-149
 enum PrefilterModeType { PREFILTER_NONE = 0, PREFILTER_LOG = 1, PREFILTER_MEANSUB = 2 };                                           // Stereo/PrefilterEnum.h:24-28
 enum CorrelationAlgorithm { VW_CORRELATION_BM = 0, VW_CORRELATION_SGM = 1, VW_CORRELATION_MGM = 2, VW_CORRELATION_FINAL_MGM = 3 };
+enum PyramidSubpixelView_Algorithm {                                                                 // Stereo/SubpixelView.h:35-40
+  SUBPIXEL_LUCAS_KANADE = 0, SUBPIXEL_FAST_AFFINE = 1, SUBPIXEL_BAYES_EM = 2, SUBPIXEL_PHASE = 3 };
 }  // namespace stereo
 }  // namespace vw

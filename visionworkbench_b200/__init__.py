@@ -4,4 +4,4 @@ SeparableConvolutionView pyramid feeder).  Product code: hand-written sm_100a ke
 reached through the C ABI of include/vwb200.h.  No CPU path, no oracle imports.
 """
 from .api import *  # noqa: F401,F403
-from .api import lib, device_count, kernel_launches, last_k1_stats  # noqa: F401
+from .api import lib, device_count, kernel_launches, last_k1_stats, last_subpixel_stats  # noqa: F401

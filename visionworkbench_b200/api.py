@@ -29,6 +29,8 @@ PREFILTER_NONE, PREFILTER_LOG, PREFILTER_MEANSUB = 0, 1, 2
 VW_CORRELATION_BM, VW_CORRELATION_SGM, VW_CORRELATION_MGM, VW_CORRELATION_FINAL_MGM = 0, 1, 2, 3
 # SemiGlobalMatcher::SgmSubpixelMode (Stereo/SGM.h:93-99)
 SUBPIXEL_NONE, SUBPIXEL_PARABOLA, SUBPIXEL_LINEAR, SUBPIXEL_POLY4, SUBPIXEL_COSINE, SUBPIXEL_LC_BLEND = 0, 1, 2, 3, 4, 5
+# PyramidSubpixelView_Algorithm (Stereo/SubpixelView.h:35-40)
+SUBPIXEL_LUCAS_KANADE, SUBPIXEL_FAST_AFFINE, SUBPIXEL_BAYES_EM, SUBPIXEL_PHASE = 0, 1, 2, 3
 
 
 class VwError(RuntimeError):
@@ -109,6 +111,9 @@ def lib():
                                                    C.POINTER(I), C.POINTER(I), I, P]
         L.vwb200_sgm_disp_bounds.argtypes = [C.POINTER(SgmParams), P, I, I, Z, P, Z, P, I, I, Z, I, I, P, I, P]
         L.vwb200_parabola_subpixel.argtypes = [P, I, I, P, Z, P, I, I, Z, I, I, I, F, I, I, I, I, P, Z, I, P]
+        L.vwb200_pyramid_subpixel.argtypes = [P, I, I, P, Z, P, I, I, Z, I, I, I, F, I, I, I, I, P, Z, I, P, I, I]
+        L.vwb200_subpixel_refine.argtypes = [I, P, I, I, Z, P, Z, P, I, I, Z, I, I, I, I, I, I, I, I, I, P]
+        L.vwb200_last_subpixel_stats.argtypes = [C.POINTER(SubpixelStats)]
         L.vwb200_cross_corr_consistency_check.argtypes = [P, I, I, Z, P, I, I, Z, F, I, P]
         L.vwb200_rm_outliers_using_thresh.argtypes = [P, I, I, I, I, D, D, P, I, P]
         L.vwb200_disparity_cleanup_using_thresh.argtypes = [P, I, I, I, I, D, D, P, I, P]
@@ -146,6 +151,20 @@ def last_k1_stats():
     s = K1Stats()
     lib().vwb200_last_k1_stats(C.byref(s))
     return {"path": "exact-int" if s.path == 0 else "general-fp64", "launches": s.launches, "kernel_ms": s.kernel_ms}
+
+
+class SubpixelStats(C.Structure):
+    _fields_ = [("levels", C.c_longlong), ("fixpoint_rounds", C.c_longlong), ("pixels", C.c_longlong),
+                ("pixels_reevaluated", C.c_longlong), ("window_evaluations", C.c_longlong), ("lane_slots", C.c_longlong)]
+
+
+def last_subpixel_stats():
+    """Counters of this thread's last sub-pixel refinement call (vwb200_last_subpixel_stats)."""
+    s = SubpixelStats()
+    _check(lib().vwb200_last_subpixel_stats(C.byref(s)))
+    d = {k: getattr(s, k) for k, _ in SubpixelStats._fields_}
+    d["simt_efficiency"] = s.window_evaluations / s.lane_slots if s.lane_slots else 0.0
+    return d
 
 
 def _is_torch(x):
@@ -401,6 +420,112 @@ class ParabolaSubpixelView:
 def parabola_subpixel(disparity, left_image, right_image, prefilter_mode, prefilter_width, kernel_size):
     """vw::stereo::parabola_subpixel (Stereo/ParabolaSubpixelView.h:111-117)."""
     return ParabolaSubpixelView(disparity, left_image, right_image, prefilter_mode, prefilter_width, kernel_size)
+
+
+class PyramidSubpixelView:
+    """vw::stereo::PyramidSubpixelView (Stereo/SubpixelView.h:42-150, .cc:33-224): lazy view refining a
+    PixelMask<Vector2f> disparity (float32 (rows, cols, 3) triples, same size as the left image) by iterative
+    Lucas-Kanade, affine or Bayes-EM affine sub-pixel correlation over an image pyramid."""
+
+    def __init__(self, disparity, left_image, right_image, prefilter_mode, prefilter_width, kernel_size,
+                 max_pyramid_levels, algorithm, phase_subpixel_accuracy=20):
+        self._d = _np(disparity, np.float32)
+        self._l, self._r = _np(left_image, np.float32), _np(right_image, np.float32)
+        if self._d.shape[:2] != self._l.shape or self._d.ndim != 3 or self._d.shape[2] != 3:
+            raise ArgumentErr("SubpixelView: Disparity image must match left image.")
+        self._mode, self._width, self._k = int(prefilter_mode), float(prefilter_width), (int(kernel_size[0]), int(kernel_size[1]))
+        self._levels, self._alg = int(max_pyramid_levels), int(algorithm)
+        self._phase_accuracy = int(phase_subpixel_accuracy)
+
+    def cols(self):
+        return self._l.shape[1]
+
+    def rows(self):
+        return self._l.shape[0]
+
+    def planes(self):
+        return 1
+
+    def __call__(self, i, j, p=0):
+        raise NoImplErr("PyramidSubpixelView::operator() is not implemented.")
+
+    def rasterize(self, dest=None, bbox=None):
+        b = _bbox(bbox) if bbox is not None else (0, 0, self.cols(), self.rows())
+        w, h = b[2] - b[0], b[3] - b[1]
+        if dest is None:
+            dest = np.empty((h, w, 3), np.float32)
+        _check(lib().vwb200_pyramid_subpixel(self._d.ctypes.data, self.cols(), self.rows(), self._l.ctypes.data, self._l.shape[1],
+                                             self._r.ctypes.data, self._r.shape[1], self._r.shape[0], self._r.shape[1],
+                                             self._k[0], self._k[1], self._mode, self._width, b[0], b[1], b[2], b[3],
+                                             dest.ctypes.data, dest.strides[0] // 12, 0, None, self._levels, self._alg))
+        return dest
+
+    prerasterize = rasterize
+
+
+def lk_subpixel(disparity, left_image, right_image, prefilter_mode, prefilter_width, kernel_size, max_pyramid_levels=2):
+    """vw::stereo::lk_subpixel (Stereo/SubpixelView.h:117-125)."""
+    return PyramidSubpixelView(disparity, left_image, right_image, prefilter_mode, prefilter_width, kernel_size,
+                               max_pyramid_levels, SUBPIXEL_LUCAS_KANADE)
+
+
+def affine_subpixel(disparity, left_image, right_image, prefilter_mode, prefilter_width, kernel_size, max_pyramid_levels=2):
+    """vw::stereo::affine_subpixel (Stereo/SubpixelView.h:127-135)."""
+    return PyramidSubpixelView(disparity, left_image, right_image, prefilter_mode, prefilter_width, kernel_size,
+                               max_pyramid_levels, SUBPIXEL_FAST_AFFINE)
+
+
+def bayes_em_subpixel(disparity, left_image, right_image, prefilter_mode, prefilter_width, kernel_size, max_pyramid_levels=2):
+    """vw::stereo::bayes_em_subpixel (Stereo/SubpixelView.h:137-145)."""
+    return PyramidSubpixelView(disparity, left_image, right_image, prefilter_mode, prefilter_width, kernel_size,
+                               max_pyramid_levels, SUBPIXEL_BAYES_EM)
+
+
+def _subpixel_refine(algorithm, disparity_map, left_image, right_image, kern_width, kern_height, region_of_interest,
+                     do_horizontal_subpixel, do_vertical_subpixel):
+    roi = _bbox(region_of_interest)
+    if _is_torch(disparity_map):
+        import torch
+        d = disparity_map.detach().clone().float().contiguous()
+        l, r = left_image.contiguous().float(), right_image.contiguous().float()
+        if tuple(d.shape) != (l.shape[0], l.shape[1], 3):
+            raise ArgumentErr("subpixel_correlation: left image and disparity map do not have the same dimensions.")
+        _check(lib().vwb200_subpixel_refine(algorithm, d.data_ptr(), l.shape[1], l.shape[0], l.shape[1], l.data_ptr(), l.stride(0),
+                                            r.data_ptr(), r.shape[1], r.shape[0], r.stride(0), kern_width, kern_height,
+                                            roi[0], roi[1], roi[2], roi[3], int(bool(do_horizontal_subpixel)),
+                                            int(bool(do_vertical_subpixel)), 1, _stream_ptr()))
+        return d
+    d = np.array(disparity_map, dtype=np.float32, order="C", copy=True)
+    l, r = _np(left_image, np.float32), _np(right_image, np.float32)
+    if d.shape != (l.shape[0], l.shape[1], 3):
+        raise ArgumentErr("subpixel_correlation: left image and disparity map do not have the same dimensions.")
+    _check(lib().vwb200_subpixel_refine(algorithm, d.ctypes.data, l.shape[1], l.shape[0], l.shape[1], l.ctypes.data, l.shape[1],
+                                        r.ctypes.data, r.shape[1], r.shape[0], r.shape[1], kern_width, kern_height,
+                                        roi[0], roi[1], roi[2], roi[3], int(bool(do_horizontal_subpixel)),
+                                        int(bool(do_vertical_subpixel)), 0, None))
+    return d
+
+
+def subpixel_optimized_LK_2d(disparity_map, left_image, right_image, kern_width, kern_height, region_of_interest,
+                             do_horizontal_subpixel=True, do_vertical_subpixel=True):
+    """vw::stereo::subpixel_optimized_LK_2d (Stereo/Correlate.h:95-104).  The reference refines disparity_map in
+    place; this returns the refined copy (numpy in, numpy out; torch CUDA in, torch CUDA out)."""
+    return _subpixel_refine(SUBPIXEL_LUCAS_KANADE, disparity_map, left_image, right_image, kern_width, kern_height,
+                            region_of_interest, do_horizontal_subpixel, do_vertical_subpixel)
+
+
+def subpixel_optimized_affine_2d(disparity_map, left_image, right_image, kern_width, kern_height, region_of_interest,
+                                 do_horizontal_subpixel=True, do_vertical_subpixel=True, verbose=False):
+    """vw::stereo::subpixel_optimized_affine_2d (Stereo/Correlate.h:74-83); returns the refined copy."""
+    return _subpixel_refine(SUBPIXEL_FAST_AFFINE, disparity_map, left_image, right_image, kern_width, kern_height,
+                            region_of_interest, do_horizontal_subpixel, do_vertical_subpixel)
+
+
+def subpixel_optimized_affine_2d_EM(disparity_map, left_image, right_image, kern_width, kern_height, region_of_interest,
+                                    do_horizontal_subpixel=True, do_vertical_subpixel=True, verbose=False):
+    """vw::stereo::subpixel_optimized_affine_2d_EM (Stereo/Correlate.h:63-72); returns the refined copy."""
+    return _subpixel_refine(SUBPIXEL_BAYES_EM, disparity_map, left_image, right_image, kern_width, kern_height,
+                            region_of_interest, do_horizontal_subpixel, do_vertical_subpixel)
 
 
 class BBox2i:

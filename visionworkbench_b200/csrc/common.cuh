@@ -181,6 +181,15 @@ int log_region_launch(const float* g, int gw, int gx0, int gy0, int iw, int ih, 
 int parabola_launch(const float* disp, int cols, int bx0, int by0, int bw, int bh, const float* L, int lw, const float* R, int rw,
                     int srx0, int sry0, int kx, int ky, float* out, cudaStream_t st);
 
+// ---- K6 PyramidSubpixelView (k6_subpixel.cu) ------------------------------------------------------------
+int k6_range_launch(const float* disp, int cols, int bx0, int by0, int bw, int bh, int* d_r5, cudaStream_t st);
+int k6_disp_crop_launch(const float* disp, int cols, int rows, int x0, int y0, int w, int h, float tx, float ty, float* out, cudaStream_t st);
+int k6_disp_out_launch(const float* patch, int pw, int ox, int oy, float tx, float ty, int w, int h, float* out, ptrdiff_t opitch, cudaStream_t st);
+int k6_level_run(int alg, float* disp, const float* L, int w, int h, const float* R, int rw, int rh, int kx, int ky,
+                 int rx0, int ry0, int rx1, int ry1, Arena& ar, cudaStream_t st, vwb200_subpixel_stats* stats);
+int k6_pyramid_run(int alg, float* D, const float* L, const float* R, int pw, int ph, int kx, int ky, int bw, int bh, int levels,
+                   Arena& ar, cudaStream_t st, vwb200_subpixel_stats* stats);
+
 // ---- host-side restatement-free logic -----------------------------------------------------------
 struct Box { int x0, y0, x1, y1; };
 struct HostZone { Box img; Box disp; };

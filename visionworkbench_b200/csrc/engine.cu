@@ -1312,6 +1312,107 @@ int vwb200_parabola_subpixel(const float* disparity, int cols, int rows, const f
   return VWB200_OK;
 }
 
+// ---- K6: PyramidSubpixelView and the level functions -------------------------------------------------------------
+static thread_local vwb200_subpixel_stats t_subpixel_stats = {0, 0, 0, 0, 0, 0};
+
+int vwb200_last_subpixel_stats(vwb200_subpixel_stats* out) { if (!out) return VWB200_EARG; *out = t_subpixel_stats; return VWB200_OK; }
+
+static int subpixel_check_algorithm(int algorithm, const char* who) {
+  if (algorithm == VWB200_SUBPIXEL_PHASE) { set_error("%s: SUBPIXEL_PHASE is not implemented", who); return VWB200_ENOIMPL; }
+  if (algorithm < VWB200_SUBPIXEL_LUCAS_KANADE || algorithm > VWB200_SUBPIXEL_BAYES_EM) {
+    set_error("%s: invalid algorithm %d", who, algorithm);
+    return VWB200_ENOIMPL;
+  }
+  return VWB200_OK;
+}
+
+int vwb200_pyramid_subpixel(const float* disparity, int cols, int rows, const float* left, ptrdiff_t lpitch,
+                            const float* right, int rcols, int rrows, ptrdiff_t rpitch, int kx, int ky,
+                            int prefilter_mode, float prefilter_width, int x0, int y0, int x1, int y1,
+                            float* dest, ptrdiff_t dest_pitch, int on_device, void* stream,
+                            int max_pyramid_levels, int algorithm) {
+  t_subpixel_stats = vwb200_subpixel_stats{0, 0, 0, 0, 0, 0};
+  if (!disparity || !left || !right || !dest) { set_error("pyramid_subpixel: null pointer"); return VWB200_EARG; }
+  if (x1 <= x0 || y1 <= y0 || x0 < 0 || y0 < 0 || x1 > cols || y1 > rows) { set_error("pyramid_subpixel: bbox outside the disparity image"); return VWB200_EARG; }
+  if (kx % 2 != 1 || ky % 2 != 1 || kx < 3 || ky < 3) { set_error("pyramid_subpixel: kernel size must be odd and >= 3"); return VWB200_EARG; }
+  if (prefilter_mode < VWB200_PREFILTER_NONE || prefilter_mode > VWB200_PREFILTER_MEANSUB) { set_error("unknown prefilter mode %d", prefilter_mode); return VWB200_EARG; }
+  VWB_TRY(subpixel_check_algorithm(algorithm, "pyramid_subpixel"));
+  const int levels = max_pyramid_levels < 0 ? 0 : max_pyramid_levels;
+  VWB_TRY(ensure_device());
+  StreamGuard sg; VWB_TRY(sg.init(stream, on_device));
+  cudaStream_t st = sg.st;
+  {
+    Arena ar(st);
+    const int bw = x1 - x0, bh = y1 - y0;
+    const float *dd, *dl, *dr; ptrdiff_t p0, p1, p2;
+    VWB_TRY(stage_in(disparity, cols * 3, rows, (ptrdiff_t)cols * 3, on_device, ar, st, &dd, &p0));
+    VWB_TRY(stage_in(left, cols, rows, lpitch, on_device, ar, st, &dl, &p1));
+    VWB_TRY(stage_in(right, rcols, rrows, rpitch, on_device, ar, st, &dr, &p2));
+    // get_disparity_range over the bbox crop: the only host round trip of the pipeline
+    int* d_r; int hr[5];
+    VWB_TRY(ar.alloc(&d_r, 5));
+    VWB_TRY(k6_range_launch(dd, cols, x0, y0, bw, bh, d_r, st));
+    VWB_CUDA(cudaMemcpyAsync(hr, d_r, sizeof(hr), cudaMemcpyDeviceToHost, st));
+    VWB_CUDA(cudaStreamSynchronize(st));
+    if (hr[4]) { set_error("pyramid_subpixel: disparity values in the bbox must be finite and below 2^24 in magnitude"); return VWB200_EARG; }
+    // SubpixelView.cc:45-61: right = bbox + range, left widened to the right's size, both grown by the kernel size
+    const Box rreg{x0 + hr[0] - kx, y0 + hr[1] - ky, x1 + hr[2] + kx, y1 + hr[3] + ky};
+    const int pw = rreg.x1 - rreg.x0, ph = rreg.y1 - rreg.y0;
+    const Box lreg{x0 - kx, y0 - ky, x0 - kx + pw, y0 - ky + ph};
+    float *Lf, *Rf, *D;
+    VWB_TRY(filtered_region(ImgF{dl, cols, rows, p1}, prefilter_mode, prefilter_width, lreg, &Lf, ar, st));
+    VWB_TRY(filtered_region(ImgF{dr, rcols, rrows, p2}, prefilter_mode, prefilter_width, rreg, &Rf, ar, st));
+    VWB_TRY(ar.alloc(&D, (size_t)pw * ph * 3));
+    VWB_TRY(k6_disp_crop_launch(dd, cols, rows, lreg.x0, lreg.y0, pw, ph, (float)hr[0], (float)hr[1], D, st));
+    VWB_TRY(k6_pyramid_run(algorithm, D, Lf, Rf, pw, ph, kx, ky, bw, bh, levels, ar, st, &t_subpixel_stats));
+    float* dout = dest;
+    ptrdiff_t opitch = dest_pitch;
+    if (!on_device) { VWB_TRY(ar.alloc(&dout, (size_t)bw * bh * 3)); opitch = bw; }
+    VWB_TRY(k6_disp_out_launch(D, pw, kx, ky, (float)hr[0], (float)hr[1], bw, bh, dout, opitch, st));
+    if (dout != dest)
+      VWB_CUDA(cudaMemcpy2DAsync(dest, (size_t)dest_pitch * 12, dout, (size_t)bw * 12, (size_t)bw * 12, bh, cudaMemcpyDeviceToHost, st));
+    VWB_CUDA(cudaStreamSynchronize(st));
+  }
+  return VWB200_OK;
+}
+
+int vwb200_subpixel_refine(int algorithm, float* disparity, int cols, int rows, ptrdiff_t dpitch,
+                           const float* left, ptrdiff_t lpitch, const float* right, int rcols, int rrows, ptrdiff_t rpitch,
+                           int kx, int ky, int x0, int y0, int x1, int y1, int do_h, int do_v, int on_device, void* stream) {
+  t_subpixel_stats = vwb200_subpixel_stats{0, 0, 0, 0, 0, 0};
+  if (!disparity || !left || !right) { set_error("subpixel_refine: null pointer"); return VWB200_EARG; }
+  if (cols <= 0 || rows <= 0 || rcols <= 0 || rrows <= 0) { set_error("subpixel_refine: empty image"); return VWB200_EARG; }
+  if (kx % 2 != 1 || ky % 2 != 1 || kx < 3 || ky < 3) { set_error("subpixel_refine: kernel size must be odd and >= 3"); return VWB200_EARG; }
+  VWB_TRY(subpixel_check_algorithm(algorithm, "subpixel_refine"));
+  if (!do_h && !do_v) return VWB200_OK;                                            // Correlate.cc:512, :861, :1213
+  VWB_TRY(ensure_device());
+  StreamGuard sg; VWB_TRY(sg.init(stream, on_device));
+  cudaStream_t st = sg.st;
+  {
+    Arena ar(st);
+    const float *dl, *dr; ptrdiff_t p1, p2;
+    VWB_TRY(stage_in(left, cols, rows, lpitch, on_device, ar, st, &dl, &p1));
+    VWB_TRY(stage_in(right, rcols, rrows, rpitch, on_device, ar, st, &dr, &p2));
+    float *D, *L = const_cast<float*>(dl), *R = const_cast<float*>(dr);
+    VWB_TRY(ar.alloc(&D, (size_t)cols * rows * 3));
+    VWB_CUDA(cudaMemcpy2DAsync(D, (size_t)cols * 12, disparity, (size_t)dpitch * 12, (size_t)cols * 12, rows,
+                               on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
+    if (p1 != cols) {
+      VWB_TRY(ar.alloc(&L, (size_t)cols * rows));
+      VWB_CUDA(cudaMemcpy2DAsync(L, (size_t)cols * 4, dl, (size_t)p1 * 4, (size_t)cols * 4, rows, cudaMemcpyDeviceToDevice, st));
+    }
+    if (p2 != rcols) {
+      VWB_TRY(ar.alloc(&R, (size_t)rcols * rrows));
+      VWB_CUDA(cudaMemcpy2DAsync(R, (size_t)rcols * 4, dr, (size_t)p2 * 4, (size_t)rcols * 4, rrows, cudaMemcpyDeviceToDevice, st));
+    }
+    VWB_TRY(k6_level_run(algorithm, D, L, cols, rows, R, rcols, rrows, kx, ky, x0, y0, x1, y1, ar, st, &t_subpixel_stats));
+    VWB_CUDA(cudaMemcpy2DAsync(disparity, (size_t)dpitch * 12, D, (size_t)cols * 12, (size_t)cols * 12, rows,
+                               on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, st));
+    VWB_CUDA(cudaStreamSynchronize(st));
+  }
+  return VWB200_OK;
+}
+
 int vwb200_subsample_mask_by_two(const uint8_t* in, int w, int h, ptrdiff_t pitch, uint8_t* out, ptrdiff_t opitch, int on_device, void* stream) {
   if (!in || !out || w <= 0 || h <= 0) { set_error("subsample_mask_by_two: bad arguments"); return VWB200_EARG; }
   VWB_TRY(ensure_device());
