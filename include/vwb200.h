@@ -163,6 +163,28 @@ typedef struct {
 int vwb200_last_subpixel_stats(vwb200_subpixel_stats* out);
 
 /* ---------------------------------------------------------------------------------------------
+ * vw::stereo::CorrEval::prerasterize(bbox) (src/vw/Stereo/CorrEval.h:56-129, CorrEval.cc:139-317): the quality of a
+ * float disparity at every sampled pixel of bbox = [x0,x1) x [y0,y1), as the NCC of the kx x ky patches around the
+ * left pixel and the right position pixel + disparity (bilinear unless round_to_int), the mean of the two patch
+ * standard deviations, or a localisation sigma from the curvature of the NCC peak.
+ * left: lw x lh, right: rw x rh PixelMask<float> = {value, valid} float pairs (pitch in pixels); disparity: lw x lh
+ * PixelMask<Vector2f> triples (dpitch in pixels); dest: (x1-x0) x (y1-y0) pairs (dest_pitch in pixels).  Pixels that
+ * are not sampled, whose disparity is invalid or whose metric fails are {0, invalid}.
+ * VWB200_EARG: a kernel that is not positive and odd, an unknown metric, sample_rate < 1, a bbox outside the left
+ * image, a prefilter_kernel_width whose padding ceil(w) + 5 is NaN, negative or above 2^20, or a sampled valid
+ * disparity in the bbox that is NaN, infinite or of magnitude >= 2^24 (dest is then left untouched).
+ * Bit-identical to the sequential reference order (DESIGN.md section K7).  The call synchronises the stream.
+ * ------------------------------------------------------------------------------------------- */
+#define VWB200_CORR_EVAL_NCC                0
+#define VWB200_CORR_EVAL_STDDEV             1
+#define VWB200_CORR_EVAL_PARABOLA_CURVATURE 2
+#define VWB200_CORR_EVAL_CRAMER_RAO         3
+int vwb200_corr_eval(const float* left, int lw, int lh, ptrdiff_t lpitch, const float* right, int rw, int rh, ptrdiff_t rpitch,
+                     const float* disparity, ptrdiff_t dpitch, int kx, int ky, int metric, int sample_rate, int round_to_int,
+                     float prefilter_kernel_width, int x0, int y0, int x1, int y1, float* dest, ptrdiff_t dest_pitch,
+                     int on_device, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * vw::stereo::calc_disparity_sgm (src/vw/Stereo/SGM.cc:167-230, SGM.h:361-376) ->
  * SemiGlobalMatcher::semi_global_matching_func (:2387-2448): u8_convert, (ternary) census costs for kernel 3/5/7/9,
  * per-pixel search boxes, SGM or MGM accumulation along 8 directions, integer winner with the reference's tie

@@ -9,6 +9,7 @@
 //   PixelGray<T>, PixelMask<T>  Image/PixelTypes.h, Image/PixelMask.h:48-160  (child + valid channel)
 //   ImageViewBase<ImplT>        Image/ImageViewBase.h:57-122   (CRTP base)
 //   ImageView<PixelT>           Image/ImageView.h:67-297       (shared buffer, cols/rows, operator(), set_size)
+//   ImageViewRef<PixelT>        Image/ImageViewRef.h           (any view behind one pixel type; held rasterised here)
 //   CropView<ImageT>            Image/Manipulation.h:82-146
 //   vw::rasterize               Image/ImageViewBase.h:283-316
 //   Exception hierarchy         Core/Exception.h:201-253
@@ -129,6 +130,18 @@ public:
   }
   typedef ImageView prerasterize_type;
   prerasterize_type prerasterize(BBox2i const&) const { return *this; }
+};
+
+// Image/ImageViewRef.h: a view of any type behind one pixel type.  The stand-in holds the view rasterised into an
+// ImageView, which is what a consumer that rasterises its inputs (the shims) observes.
+template <class PixelT> class ImageViewRef : public ImageViewBase<ImageViewRef<PixelT>> {
+  ImageView<PixelT> m_view;
+public:
+  typedef PixelT pixel_type; typedef PixelT result_type;
+  template <class ViewT> ImageViewRef(ImageViewBase<ViewT> const& view) : m_view(view) {}
+  int32 cols() const { return m_view.cols(); } int32 rows() const { return m_view.rows(); } int32 planes() const { return m_view.planes(); }
+  result_type operator()(int32 c, int32 r, int32 p = 0) const { return m_view(c, r, p); }
+  template <class DestT> void rasterize(DestT const& dest, BBox2i const& bbox) const { m_view.rasterize(dest, bbox); }
 };
 
 template <class ImageT> class CropView : public ImageViewBase<CropView<ImageT>> {             // Image/Manipulation.h:82-146

@@ -31,6 +31,8 @@ VW_CORRELATION_BM, VW_CORRELATION_SGM, VW_CORRELATION_MGM, VW_CORRELATION_FINAL_
 SUBPIXEL_NONE, SUBPIXEL_PARABOLA, SUBPIXEL_LINEAR, SUBPIXEL_POLY4, SUBPIXEL_COSINE, SUBPIXEL_LC_BLEND = 0, 1, 2, 3, 4, 5
 # PyramidSubpixelView_Algorithm (Stereo/SubpixelView.h:35-40)
 SUBPIXEL_LUCAS_KANADE, SUBPIXEL_FAST_AFFINE, SUBPIXEL_BAYES_EM, SUBPIXEL_PHASE = 0, 1, 2, 3
+# CorrEval metrics (Stereo/CorrEval.h:88-90), VWB200_CORR_EVAL_*
+CORR_EVAL_METRICS = {"ncc": 0, "stddev": 1, "parabola_curvature": 2, "cramer_rao": 3}
 
 
 class VwError(RuntimeError):
@@ -114,6 +116,7 @@ def lib():
         L.vwb200_pyramid_subpixel.argtypes = [P, I, I, P, Z, P, I, I, Z, I, I, I, F, I, I, I, I, P, Z, I, P, I, I]
         L.vwb200_subpixel_refine.argtypes = [I, P, I, I, Z, P, Z, P, I, I, Z, I, I, I, I, I, I, I, I, I, P]
         L.vwb200_last_subpixel_stats.argtypes = [C.POINTER(SubpixelStats)]
+        L.vwb200_corr_eval.argtypes = [P, I, I, Z, P, I, I, Z, P, Z, I, I, I, I, I, F, I, I, I, I, P, Z, I, P]
         L.vwb200_cross_corr_consistency_check.argtypes = [P, I, I, Z, P, I, I, Z, F, I, P]
         L.vwb200_rm_outliers_using_thresh.argtypes = [P, I, I, I, I, D, D, P, I, P]
         L.vwb200_disparity_cleanup_using_thresh.argtypes = [P, I, I, I, I, D, D, P, I, P]
@@ -526,6 +529,98 @@ def subpixel_optimized_affine_2d_EM(disparity_map, left_image, right_image, kern
     """vw::stereo::subpixel_optimized_affine_2d_EM (Stereo/Correlate.h:63-72); returns the refined copy."""
     return _subpixel_refine(SUBPIXEL_BAYES_EM, disparity_map, left_image, right_image, kern_width, kern_height,
                             region_of_interest, do_horizontal_subpixel, do_vertical_subpixel)
+
+
+def _masked(img):
+    """PixelMask<float> raster: (rows, cols, 2) float32 {value, valid}; a 2-D image is all valid."""
+    if _is_torch(img):
+        import torch
+        t = img.detach().float()
+        if t.dim() == 2:
+            t = torch.stack([t, torch.ones_like(t)], dim=-1)
+        return t.contiguous()
+    a = np.asarray(img, dtype=np.float32)
+    if a.ndim == 2:
+        a = np.stack([a, np.ones_like(a)], axis=-1)
+    return np.ascontiguousarray(a)
+
+
+class CorrEval:
+    """vw::stereo::CorrEval (Stereo/CorrEval.h:56-129, CorrEval.cc:139-317): lazy view of the quality of a float disparity
+    at every pixel -- "ncc", "stddev", "parabola_curvature" or "cramer_rao" over kernel_size windows, at the pixels whose
+    coordinates in the rasterised bbox are multiples of sample_rate.  Images are float32 (rows, cols, 2) {value, valid}
+    or 2-D float32 (all valid); the disparity is (rows, cols, 3) {dx, dy, valid} of the left image's size.  rasterize()
+    returns (rows, cols, 2) {value, valid}: numpy for numpy inputs, torch CUDA tensors (on the current stream) for
+    torch CUDA inputs.  prefilter_mode is accepted and unused, as in the reference; prefilter_kernel_width sets the crop
+    padding, which moves the right crop's origin and hence the float rounding of the bilinear weights."""
+
+    def __init__(self, left, right, disp, kernel_size, metric, sample_rate, round_to_int, prefilter_mode=0,
+                 prefilter_kernel_width=0.0):
+        self._torch = _is_torch(disp)
+        if any(_is_torch(x) != self._torch or (self._torch and not x.is_cuda) for x in (left, right, disp)):
+            raise ArgumentErr("CorrEval: the images and the disparity must all be numpy arrays or all torch CUDA tensors.")
+        self._l, self._r = _masked(left), _masked(right)
+        if self._torch:
+            self._d = disp.detach().float().contiguous()
+        else:
+            self._d = _np(disp, np.float32)
+        if tuple(self._d.shape[:2]) != tuple(self._l.shape[:2]) or self._d.ndim != 3 or self._d.shape[2] != 3:
+            raise ArgumentErr("CorrEval: Left image and disparity must have the same dimensions.")
+        self._k = (int(kernel_size[0]), int(kernel_size[1]))
+        if not all(k > 0 and k % 2 == 1 for k in self._k):
+            raise ArgumentErr("CorrEval: The kernel dimensions must be positive and odd.")
+        if metric not in CORR_EVAL_METRICS:
+            raise ArgumentErr(f"CorrEval: Invalid metric: {metric}.")
+        self._metric = CORR_EVAL_METRICS[metric]
+        self._sample_rate, self._round = int(sample_rate), int(bool(round_to_int))
+        self._prefilter_mode, self._pkw = int(prefilter_mode), float(prefilter_kernel_width)
+
+    def cols(self):
+        return self._l.shape[1]
+
+    def rows(self):
+        return self._l.shape[0]
+
+    def planes(self):
+        return 1
+
+    def __call__(self, i, j, p=0):
+        raise NoImplErr("CorrEval::operator() is not implemented.")
+
+    def rasterize(self, dest=None, bbox=None):
+        b = _bbox(bbox) if bbox is not None else (0, 0, self.cols(), self.rows())
+        w, h = b[2] - b[0], b[3] - b[1]
+        l, r, d = self._l, self._r, self._d
+        shape = (max(h, 0), max(w, 0), 2)
+        if self._torch:
+            import torch
+            if dest is None:
+                dest = torch.empty(shape, dtype=torch.float32, device=d.device)
+            elif not (_is_torch(dest) and dest.is_cuda and dest.device == d.device and dest.dtype == torch.float32
+                      and tuple(dest.shape) == shape and dest.stride(2) == 1 and dest.stride(1) == 2 and dest.stride(0) % 2 == 0):
+                raise ArgumentErr(f"CorrEval: dest must be a float32 CUDA tensor of shape {shape} on {d.device} "
+                                  "with contiguous pixels")
+            ptr = lambda t: t.data_ptr()
+            pitch, on_device, stream = dest.stride(0) // 2, 1, _stream_ptr()
+        else:
+            if dest is None:
+                dest = np.empty(shape, np.float32)
+            elif not (isinstance(dest, np.ndarray) and dest.dtype == np.float32 and dest.shape == shape and dest.flags.writeable
+                      and dest.strides[2] == 4 and dest.strides[1] == 8 and dest.strides[0] % 8 == 0):
+                raise ArgumentErr(f"CorrEval: dest must be a writable float32 numpy array of shape {shape} with contiguous pixels")
+            ptr = lambda a: a.ctypes.data
+            pitch, on_device, stream = dest.strides[0] // 8, 0, None
+        _check(lib().vwb200_corr_eval(ptr(l), l.shape[1], l.shape[0], l.shape[1], ptr(r), r.shape[1], r.shape[0], r.shape[1],
+                                      ptr(d), d.shape[1], self._k[0], self._k[1], self._metric, self._sample_rate, self._round,
+                                      self._pkw, b[0], b[1], b[2], b[3], ptr(dest), pitch, on_device, stream))
+        return dest
+
+    prerasterize = rasterize
+
+
+def corr_eval(left, right, disp, kernel_size, metric, sample_rate, round_to_int, prefilter_mode=0, prefilter_kernel_width=0.0):
+    """vw::stereo::corr_eval (Stereo/CorrEval.h:117-128)."""
+    return CorrEval(left, right, disp, kernel_size, metric, sample_rate, round_to_int, prefilter_mode, prefilter_kernel_width)
 
 
 class BBox2i:

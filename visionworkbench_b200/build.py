@@ -13,7 +13,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(ROOT, "build", "obj")
 SO = os.path.join(HERE, "libvwb200.so")
-SOURCES = ["engine.cu", "k1_generic.cu", "k1_zone_int.cu", "k1_fast.cu", "k1_screen.cu", "k2_pyramid.cu", "k34_filters.cu", "k5_sgm.cu", "k5_sgm_paths.cu", "shard.cu", "k6_subpixel.cu"]
+SOURCES = ["engine.cu", "k1_generic.cu", "k1_zone_int.cu", "k1_fast.cu", "k1_screen.cu", "k2_pyramid.cu", "k34_filters.cu", "k5_sgm.cu", "k5_sgm_paths.cu", "shard.cu", "k6_subpixel.cu", "k7_corr_eval.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"] + os.environ.get("VWB200_NVCC_EXTRA", "").split()
 

@@ -190,6 +190,15 @@ int k6_level_run(int alg, float* disp, const float* L, int w, int h, const float
 int k6_pyramid_run(int alg, float* D, const float* L, const float* R, int pw, int ph, int kx, int ky, int bw, int bh, int levels,
                    Arena& ar, cudaStream_t st, vwb200_subpixel_stats* stats);
 
+// ---- K7 CorrEval (k7_corr_eval.cu) ------------------------------------------------------------------------
+// d_org3 = {min over the sampled valid pixels of col + floor(dx), of row + floor(dy), bad-disparity flag}
+int k7_origin_launch(const float* D, ptrdiff_t dpitch, int x0, int y0, int bw, int bh, int sample_rate, int round_to_int, int* d_org3,
+                     cudaStream_t st);
+// writes nothing when d_org3[2] is set
+int k7_corr_eval_launch(const float* L, int lw, int lh, ptrdiff_t lpitch, const float* R, int rw, int rh, ptrdiff_t rpitch,
+                        const float* D, ptrdiff_t dpitch, int x0, int y0, int bw, int bh, int kx, int ky, int metric, int sample_rate,
+                        int round_to_int, int margin, const int* d_org3, float* out, ptrdiff_t opitch, cudaStream_t st);
+
 // ---- host-side restatement-free logic -----------------------------------------------------------
 struct Box { int x0, y0, x1, y1; };
 struct HostZone { Box img; Box disp; };

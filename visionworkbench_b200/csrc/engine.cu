@@ -1413,6 +1413,52 @@ int vwb200_subpixel_refine(int algorithm, float* disparity, int cols, int rows, 
   return VWB200_OK;
 }
 
+// ---- K7: CorrEval ------------------------------------------------------------------------------------------------
+int vwb200_corr_eval(const float* left, int lw, int lh, ptrdiff_t lpitch, const float* right, int rw, int rh, ptrdiff_t rpitch,
+                     const float* disparity, ptrdiff_t dpitch, int kx, int ky, int metric, int sample_rate, int round_to_int,
+                     float prefilter_kernel_width, int x0, int y0, int x1, int y1, float* dest, ptrdiff_t dest_pitch,
+                     int on_device, void* stream) {
+  if (!left || !right || !disparity || !dest) { set_error("corr_eval: null pointer"); return VWB200_EARG; }
+  if (lw <= 0 || lh <= 0 || rw <= 0 || rh <= 0) { set_error("corr_eval: empty image"); return VWB200_EARG; }
+  if (!(kx > 0 && kx % 2 == 1 && ky > 0 && ky % 2 == 1)) { set_error("CorrEval: The kernel dimensions must be positive and odd."); return VWB200_EARG; }
+  if (metric < VWB200_CORR_EVAL_NCC || metric > VWB200_CORR_EVAL_CRAMER_RAO) { set_error("CorrEval: Invalid metric: %d.", metric); return VWB200_EARG; }
+  if (sample_rate < 1) { set_error("CorrEval: the sample rate must be at least 1"); return VWB200_EARG; }
+  if (x1 <= x0 || y1 <= y0 || x0 < 0 || y0 < 0 || x1 > lw || y1 > lh) { set_error("corr_eval: bbox outside the left image"); return VWB200_EARG; }
+  // m_extra_padding = (int)ceil(prefilter_kernel_width) + 5 (CorrEval.h:77)
+  const float pad = ceilf(prefilter_kernel_width) + 5.0f;
+  if (!(pad >= 0.0f && pad <= 1048576.0f)) { set_error("corr_eval: prefilter_kernel_width must give a padding ceil(w) + 5 in [0, 2^20]"); return VWB200_EARG; }
+  const bool curvature = metric == VWB200_CORR_EVAL_PARABOLA_CURVATURE || metric == VWB200_CORR_EVAL_CRAMER_RAO;
+  const int margin = 1 + 2 + (int)pad + (curvature ? 1 : 0);   // CorrEval.cc:205-214
+  VWB_TRY(ensure_device());
+  StreamGuard sg; VWB_TRY(sg.init(stream, on_device));
+  cudaStream_t st = sg.st;
+  const int bw = x1 - x0, bh = y1 - y0;
+  int bad = 0;
+  {
+    Arena ar(st);
+    const float *dl, *dr, *dd; ptrdiff_t pl, pr, pd;
+    VWB_TRY(stage_in(left, lw * 2, lh, lpitch * 2, on_device, ar, st, &dl, &pl));
+    VWB_TRY(stage_in(right, rw * 2, rh, rpitch * 2, on_device, ar, st, &dr, &pr));
+    VWB_TRY(stage_in(disparity, lw * 3, lh, dpitch * 3, on_device, ar, st, &dd, &pd));
+    int* d_org;
+    VWB_TRY(ar.alloc(&d_org, 3));
+    VWB_TRY(k7_origin_launch(dd, pd / 3, x0, y0, bw, bh, sample_rate, round_to_int, d_org, st));
+    float* dout = dest;
+    ptrdiff_t opitch = dest_pitch;
+    if (!on_device) { VWB_TRY(ar.alloc(&dout, (size_t)bw * bh * 2)); opitch = bw; }
+    VWB_TRY(k7_corr_eval_launch(dl, lw, lh, pl / 2, dr, rw, rh, pr / 2, dd, pd / 3, x0, y0, bw, bh, kx, ky, metric, sample_rate,
+                                round_to_int, margin, d_org, dout, opitch, st));
+    VWB_CUDA(cudaMemcpyAsync(&bad, d_org + 2, sizeof(int), cudaMemcpyDeviceToHost, st));
+    VWB_CUDA(cudaStreamSynchronize(st));
+    if (!bad && dout != dest) {
+      VWB_CUDA(cudaMemcpy2DAsync(dest, (size_t)dest_pitch * 8, dout, (size_t)bw * 8, (size_t)bw * 8, bh, cudaMemcpyDeviceToHost, st));
+      VWB_CUDA(cudaStreamSynchronize(st));
+    }
+  }
+  if (bad) { set_error("corr_eval: sampled valid disparities in the bbox must be finite and below 2^24 in magnitude"); return VWB200_EARG; }
+  return VWB200_OK;
+}
+
 int vwb200_subsample_mask_by_two(const uint8_t* in, int w, int h, ptrdiff_t pitch, uint8_t* out, ptrdiff_t opitch, int on_device, void* stream) {
   if (!in || !out || w <= 0 || h <= 0) { set_error("subsample_mask_by_two: bad arguments"); return VWB200_EARG; }
   VWB_TRY(ensure_device());
