@@ -135,7 +135,7 @@ int k1_nan_fixup_launch(int cost, ImgF left, ImgF right, const Zone* d_zones, in
 // ---- K1 fast (exact-integer path, single big zone) -------------------------------------------
 // Returns VWB200_ENOIMPL if the configuration is outside what the fast path handles.
 int k1_fast_supported(int cost, int kx, int ky, int sx, int sy, float vmin, float vmax, bool integer_valued);
-int k1_fast_launch(int cost, ImgF left, ImgF right, int W, int H, int sx, int sy, int kx, int ky, float vmin, float vmax,
+int k1_fast_launch(int cost, ImgF left, ImgF right, int W, int H, int sx, int sy, int kx, int ky, float vmin,
                    vwb200_dispi* out, ptrdiff_t opitch, void* workspace, size_t workspace_bytes, cudaStream_t st,
                    const KEvents* ev = nullptr, const struct FastOrigin* org = nullptr);
 size_t k1_fast_workspace_bytes(int W, int H, int sx, int sy, int kx, int ky);

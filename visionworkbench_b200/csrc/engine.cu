@@ -667,7 +667,7 @@ int vwb200_corr::prerasterize(Box bbox, vwb200_dispi** d_disp_out, float** d_sub
         if (k1_fast_supported(p.cost_type, kx, ky, z.sx, z.sy, tile_vmin, tile_vmax, true) == VWB200_OK) {
           const size_t wb = k1_fast_workspace_bytes(z.w, z.h, z.sx, z.sy, kx, ky);
           VWB_TRY(ar.alloc(&ws, wb));
-          VWB_TRY(k1_fast_launch(p.cost_type, a, b, z.w, z.h, z.sx, z.sy, kx, ky, tile_vmin, tile_vmax, dst + z.obase, z.opitch, ws, wb, st, nullptr, &org));
+          VWB_TRY(k1_fast_launch(p.cost_type, a, b, z.w, z.h, z.sx, z.sy, kx, ky, tile_vmin, dst + z.obase, z.opitch, ws, wb, st, nullptr, &org));
           flag = 1;
         } else if (k1_screen_supported(p.cost_type, kx, ky, z.sx, z.sy, tile_vmin, tile_vmax, true) == VWB200_OK) {
           VWB_TRY(ar.alloc(&ws, k1_screen_workspace_bytes(p.cost_type, z.w, z.h, z.sx, z.sy, kx, ky)));
@@ -920,9 +920,9 @@ static int calc_disparity_device(int cost_type, ImgF Li, ImgF Ri, int W, int H, 
     const size_t wb = k1_fast_workspace_bytes(W, H, sx, sy, kx, ky);
     unsigned char* ws;
     VWB_TRY(ar.alloc(&ws, wb));
-    VWB_TRY(k1_fast_launch(cost_type, Li, Ri, W, H, sx, sy, kx, ky, vmin, vmax, dout, dop, ws, wb, st, kev));
+    VWB_TRY(k1_fast_launch(cost_type, Li, Ri, W, H, sx, sy, kx, ky, vmin, dout, dop, ws, wb, st, kev));
     path = 0;
-  } else if (k1_screen_supported(cost_type, kx, ky, sx, sy, vmin, vmax, integer) == VWB200_OK && !getenv("VWB200_K1_GENERIC")) {
+  } else if (k1_screen_supported(cost_type, kx, ky, sx, sy, vmin, vmax, integer) == VWB200_OK) {
     unsigned char* ws;
     VWB_TRY(ar.alloc(&ws, k1_screen_workspace_bytes(cost_type, W, H, sx, sy, kx, ky)));
     VWB_TRY(k1_screen_launch(cost_type, Li, Ri, W, H, sx, sy, kx, ky, vmin, vmax, dout, dop, ws, st, kev));

@@ -22,8 +22,6 @@
 //   * pixels whose arg-best is disparity (0,0) are re-checked by a small kernel for the
 //     "every disparity gave the same cost => invalid" rule (Correlation.cc:121-133)
 #include "k1_fast_common.cuh"
-#include <cstdlib>
-#include <cstring>
 
 namespace vwb200 {
 
@@ -143,23 +141,7 @@ __device__ __forceinline__ void load_row(const uint16_t* lrow, const uint16_t* r
   for (int i = 0; i < 8; ++i) Rv[8 + i] = t[i];
 }
 
-__device__ __forceinline__ void unpack8f(const uint4 v, float (&o)[8]) {
-  o[0] = __uint_as_float(__byte_perm(v.x, 0x4B000000u, 0x7610)); o[1] = __uint_as_float(__byte_perm(v.x, 0x4B000000u, 0x7632));
-  o[2] = __uint_as_float(__byte_perm(v.y, 0x4B000000u, 0x7610)); o[3] = __uint_as_float(__byte_perm(v.y, 0x4B000000u, 0x7632));
-  o[4] = __uint_as_float(__byte_perm(v.z, 0x4B000000u, 0x7610)); o[5] = __uint_as_float(__byte_perm(v.z, 0x4B000000u, 0x7632));
-  o[6] = __uint_as_float(__byte_perm(v.w, 0x4B000000u, 0x7610)); o[7] = __uint_as_float(__byte_perm(v.w, 0x4B000000u, 0x7632));
-}
-__device__ __forceinline__ void load_row_f(const uint16_t* lrow, const uint16_t* rrow, float (&Lv)[8], float (&Rv)[16]) {
-  unpack8f(*reinterpret_cast<const uint4*>(lrow), Lv);
-  float t[8];
-  unpack8f(*reinterpret_cast<const uint4*>(rrow), t);
-#pragma unroll
-  for (int i = 0; i < 8; ++i) Rv[i] = t[i];
-  unpack8f(*reinterpret_cast<const uint4*>(rrow + 8), t);
-#pragma unroll
-  for (int i = 0; i < 8; ++i) Rv[8 + i] = t[i];
-}
-template <int KX, bool FSEED, bool FULL>
+template <int KX, bool FULL>
 __device__ __forceinline__ void fast_pass(const uint16_t* __restrict__ ltile, const uint16_t* __restrict__ rring,
                                           uint32_t* __restrict__ state, uint16_t* __restrict__ idxp,
                                           int lane, int g, int ky, int ring_slots, int rw, int ring_base, int idx_base, int row0, int nb) {
@@ -167,41 +149,19 @@ __device__ __forceinline__ void fast_pass(const uint16_t* __restrict__ ltile, co
   const uint16_t* lp = ltile + row0 * F_COLS + 8 * lane;       // + row*256            (16-byte aligned)
   const uint16_t* rp = rring + 8 * (lane + g);                 // + slot*rw            (16-byte aligned)
   int slot_new = ring_base;                                     // ring slot of right row (dy + row0 + t)
-  // ---- seed: first ky rows.  The integer main loop is bound by the ALU pipe (VABSDIFF), so the seed
-  //      rows are summed in fp32 on the otherwise idle FMA pipes (exact: sums < 2^23) and converted once.
-  if (FSEED) {
-    float Vf[8][F_B];
+  // ---- seed: first ky rows
+#pragma unroll
+  for (int a = 0; a < 8; ++a)
+#pragma unroll
+    for (int b = 0; b < F_B; ++b) V[a][b] = 0;
+  for (int t = 0; t < ky; ++t) {
+    int Lv[8], Rv[16];
+    load_row(lp + t * F_COLS, rp + slot_new * rw, Lv, Rv);
 #pragma unroll
     for (int a = 0; a < 8; ++a)
 #pragma unroll
-      for (int b = 0; b < F_B; ++b) Vf[a][b] = 0.0f;
-    for (int t = 0; t < ky; ++t) {
-      float Lv[8], Rv[16];
-      load_row_f(lp + t * F_COLS, rp + slot_new * rw, Lv, Rv);
-#pragma unroll
-      for (int a = 0; a < 8; ++a)
-#pragma unroll
-        for (int b = 0; b < F_B; ++b) Vf[a][b] = __fadd_rn(Vf[a][b], fabsf(__fsub_rn(Lv[a], Rv[a + b])));
-      if (++slot_new == ring_slots) slot_new = 0;
-    }
-#pragma unroll
-    for (int a = 0; a < 8; ++a)
-#pragma unroll
-      for (int b = 0; b < F_B; ++b) V[a][b] = (int)__float_as_uint(__fadd_rn(Vf[a][b], 8388608.0f)) - 0x4B000000;
-  } else {
-#pragma unroll
-    for (int a = 0; a < 8; ++a)
-#pragma unroll
-      for (int b = 0; b < F_B; ++b) V[a][b] = 0;
-    for (int t = 0; t < ky; ++t) {
-      int Lv[8], Rv[16];
-      load_row(lp + t * F_COLS, rp + slot_new * rw, Lv, Rv);
-#pragma unroll
-      for (int a = 0; a < 8; ++a)
-#pragma unroll
-        for (int b = 0; b < F_B; ++b) V[a][b] = __sad(Lv[a], Rv[a + b], V[a][b]);
-      if (++slot_new == ring_slots) slot_new = 0;
-    }
+      for (int b = 0; b < F_B; ++b) V[a][b] = __sad(Lv[a], Rv[a + b], V[a][b]);
+    if (++slot_new == ring_slots) slot_new = 0;
   }
   int slot_old = ring_base;
   for (int y = 0; y < F_RH; ++y) {
@@ -331,110 +291,7 @@ __device__ __forceinline__ void fast_pass_sq(const uint16_t* __restrict__ ltile,
   }
 }
 
-// ---- float variant of the pass: the same exact integers carried in fp32 ----------------------------------
-// The ALU pipe (VABSDIFF, integer min, unpack) is the bound of the integer pass; FADD runs on the FMA
-// pipes at twice the ALU rate.  Unpacking u16 -> "2^23 + x" biased floats is a single PRMT, differences
-// of biased floats are exact, and every sum stays below 2^24 (checked on the host), so the fp32 pass
-// produces the same integers.
-template <int KX>
-__device__ __forceinline__ void window_sums_f(const float (&p)[8], float (&out)[8]) {
-  const float T = p[7];
-  constexpr int MAXL = (KX - 1) / 8;
-  float W[MAXL + 1];
-  W[0] = T;
-#pragma unroll
-  for (int k = 1; k <= MAXL; ++k) W[k] = __fadd_rn(W[k - 1], __shfl_down_sync(0xffffffffu, T, k));
-#pragma unroll
-  for (int r = 0; r < 8; ++r) {
-    const int own = 8 - r;
-    if (KX <= own) {
-      out[r] = r ? __fsub_rn(p[r + KX - 1], p[r - 1]) : p[KX - 1];
-    } else {
-      const int rem = KX - own;
-      const int full = rem / 8, part = rem % 8;
-      if (part) {
-        const float q = __shfl_down_sync(0xffffffffu, p[part - 1], full + 1);
-        out[r] = r ? __fadd_rn(__fsub_rn(W[full], p[r - 1]), q) : __fadd_rn(W[full], q);
-      } else {
-        out[r] = r ? __fsub_rn(W[full], p[r - 1]) : W[full];
-      }
-    }
-  }
-}
-
-template <int KX>
-__device__ __forceinline__ void fast_pass_f(const uint16_t* __restrict__ ltile, const uint16_t* __restrict__ rring,
-                                            float* __restrict__ state, uint16_t* __restrict__ idxp,
-                                            int lane, int g, int ky, int ring_slots, int rw, int ring_base, int idx_base, int row0) {
-  float V[8][F_B];
-#pragma unroll
-  for (int a = 0; a < 8; ++a)
-#pragma unroll
-    for (int b = 0; b < F_B; ++b) V[a][b] = 0.0f;
-  const uint16_t* lp = ltile + row0 * F_COLS + 8 * lane;
-  const uint16_t* rp = rring + 8 * (lane + g);
-  int slot_new = ring_base;
-  for (int t = 0; t < ky; ++t) {
-    float Lv[8], Rv[16];
-    load_row_f(lp + t * F_COLS, rp + slot_new * rw, Lv, Rv);
-#pragma unroll
-    for (int a = 0; a < 8; ++a)
-#pragma unroll
-      for (int b = 0; b < F_B; ++b) V[a][b] = __fadd_rn(V[a][b], fabsf(__fsub_rn(Lv[a], Rv[a + b])));
-    if (++slot_new == ring_slots) slot_new = 0;
-  }
-  int slot_old = ring_base;
-  for (int y = 0; y < F_RH; ++y) {
-    if (y > 0) {
-      {
-        float Lv[8], Rv[16];
-        load_row_f(lp + (y + ky - 1) * F_COLS, rp + slot_new * rw, Lv, Rv);
-#pragma unroll
-        for (int a = 0; a < 8; ++a)
-#pragma unroll
-          for (int b = 0; b < F_B; ++b) V[a][b] = __fadd_rn(V[a][b], fabsf(__fsub_rn(Lv[a], Rv[a + b])));
-      }
-      {
-        float Lo[8], Ro[16];
-        load_row_f(lp + (y - 1) * F_COLS, rp + slot_old * rw, Lo, Ro);
-#pragma unroll
-        for (int a = 0; a < 8; ++a)
-#pragma unroll
-          for (int b = 0; b < F_B; ++b) V[a][b] = __fsub_rn(V[a][b], fabsf(__fsub_rn(Lo[a], Ro[a + b])));
-      }
-      if (++slot_new == ring_slots) slot_new = 0;
-      if (++slot_old == ring_slots) slot_old = 0;
-    }
-    float m[8];
-#pragma unroll
-    for (int b = 0; b < F_B; ++b) {
-      float p[8], o[8];
-      p[0] = V[0][b];
-#pragma unroll
-      for (int a = 1; a < 8; ++a) p[a] = __fadd_rn(p[a - 1], V[a][b]);
-      window_sums_f<KX>(p, o);
-#pragma unroll
-      for (int r = 0; r < 8; ++r) m[r] = (b == 0) ? o[r] : fminf(__fadd_rn(o[r], (float)b), m[r]);
-    }
-    float* srow = state + y * F_COLS + lane;
-    float s8[8];
-    bool improved = false;
-#pragma unroll
-    for (int r = 0; r < 8; ++r) { s8[r] = srow[r * 32]; improved |= (m[r] < s8[r]); }
-    if (improved) {
-#pragma unroll
-      for (int r = 0; r < 8; ++r) {
-        if (m[r] < s8[r]) {
-          const int bi = (int)__float_as_uint(__fadd_rn(m[r], 8388608.0f)) & 7;
-          srow[r * 32] = __fsub_rn(m[r], (float)bi);
-          idxp[y * F_COLS + r * 32 + lane] = (uint16_t)(idx_base + bi);
-        }
-      }
-    }
-  }
-}
-
-template <int KX, bool FLT, bool FSEED, bool SQ = false>
+template <int KX, bool SQ>
 __global__ void __launch_bounds__(F_THREADS, 1)
 k1_fast_abs_kernel(const uint16_t* __restrict__ L16, const uint16_t* __restrict__ R16, FastGeom G,
                    uint16_t* __restrict__ idx_scratch, vwb200_dispi* __restrict__ out, ptrdiff_t opitch,
@@ -465,7 +322,7 @@ k1_fast_abs_kernel(const uint16_t* __restrict__ L16, const uint16_t* __restrict_
       tma_load_1d(ltile, lsrc, lbytes, &bars[0]);
       tma_load_1d(rring, rsrc, (uint32_t)G.ltile_rows * rrow_bytes, &bars[0]);     // right rows y0 .. y0+ltile_rows-1 -> slots 0..
     }
-    for (int k = tid; k < F_SUBSETS * F_TH * F_COLS; k += F_THREADS) state[k] = SQ ? 0xffffffffu : (FLT ? 0x7f000000u : S_INIT);     // 1.7e38f as float bits / max key
+    for (int k = tid; k < F_SUBSETS * F_TH * F_COLS; k += F_THREADS) state[k] = SQ ? 0xffffffffu : S_INIT;     // max cost / max key
     __syncthreads();
     mbar_wait(&bars[0], ph0); ph0 ^= 1;
     uint32_t* wstate = state + ((size_t)sub * F_TH + row0) * F_COLS;       // this warp's rows of its subset plane
@@ -480,12 +337,11 @@ k1_fast_abs_kernel(const uint16_t* __restrict__ L16, const uint16_t* __restrict_
       for (int g = sub; g < ngroups; g += F_SUBSETS) {
         if (SQ) fast_pass_sq<KX>(ltile, rring, wstate, widx, lane, g, G.ky, G.ring_slots, G.rw, ring_base, (dy0 + dy) * G.sx + F_B * g, row0,
                                  min(F_B, G.sx - F_B * g));
-        else if (FLT) fast_pass_f<KX>(ltile, rring, reinterpret_cast<float*>(wstate), widx, lane, g, G.ky, G.ring_slots, G.rw, ring_base, (dy0 + dy) * G.sx + F_B * g, row0);
         else if (G.sx - F_B * g >= F_B)
-          fast_pass<KX, FSEED, true>(ltile, rring, wstate, widx, lane, g, G.ky, G.ring_slots, G.rw, ring_base, (dy0 + dy) * G.sx + F_B * g, row0, F_B);
+          fast_pass<KX, true>(ltile, rring, wstate, widx, lane, g, G.ky, G.ring_slots, G.rw, ring_base, (dy0 + dy) * G.sx + F_B * g, row0, F_B);
         else
-          fast_pass<KX, FSEED, false>(ltile, rring, wstate, widx, lane, g, G.ky, G.ring_slots, G.rw, ring_base, (dy0 + dy) * G.sx + F_B * g, row0,
-                                      G.sx - F_B * g);
+          fast_pass<KX, false>(ltile, rring, wstate, widx, lane, g, G.ky, G.ring_slots, G.rw, ring_base, (dy0 + dy) * G.sx + F_B * g, row0,
+                               G.sx - F_B * g);
       }
       if (dy + 1 < ndy) { mbar_wait(&bars[1], ph1); ph1 ^= 1; }
       __syncthreads();
@@ -559,7 +415,7 @@ __global__ void k1_fast_allequal_fixup(ImgF L, ImgF R, FastGeom g, vwb200_dispi*
   o->valid = 0;
 }
 
-int k1_fast_launch(int cost, ImgF left, ImgF right, int W, int H, int sx, int sy, int kx, int ky, float vmin, float vmax,
+int k1_fast_launch(int cost, ImgF left, ImgF right, int W, int H, int sx, int sy, int kx, int ky, float vmin,
                    vwb200_dispi* out, ptrdiff_t opitch, void* workspace, size_t workspace_bytes, cudaStream_t st,
                    const KEvents* ev, const FastOrigin* org) {
   (void)workspace_bytes;
@@ -567,14 +423,6 @@ int k1_fast_launch(int cost, ImgF left, ImgF right, int W, int H, int sx, int sy
   FastGeom g = make_geom(W, H, sx, sy, kx, ky);
   g.scale = sq ? 1 : F_B;
   if (org) { g.lox = org->lox; g.loy = org->loy; g.rox = org->rox; g.roy = org->roy; g.addx = org->addx; g.addy = org->addy; }
-  // fp32 carries the integers exactly while every window sum * 8 (+7) stays below 2^24
-  // variants: all-int (default, ALU-pipe bound), int with fp32 seeding (VWB200_K1_FAST=fseed), all-fp32 on the FMA
-  // pipes (VWB200_K1_FAST=float; issue-bound).  All three are exact; profiles/k1_fast_variants_r01.md has the numbers.
-  const char* mode = getenv("VWB200_K1_FAST");
-  const bool float_ok = (double)(vmax - vmin) * kx * ky * F_B + F_B < 16777216.0;
-  const bool fseed_ok = (double)(vmax - vmin) * ky * F_B < 8388608.0;
-  const bool use_float = float_ok && mode && !strcmp(mode, "float");
-  const bool float_seed = fseed_ok && mode && !strcmp(mode, "fseed");     // measured 3 % slower than all-int (issue-bound)
   unsigned char* ws = static_cast<unsigned char*>(workspace);
   uint16_t* L16 = reinterpret_cast<uint16_t*>(ws);
   uint16_t* R16 = L16 + (size_t)g.NS * g.lrows * F_COLS;
@@ -596,7 +444,7 @@ int k1_fast_launch(int cost, ImgF left, ImgF right, int W, int H, int sx, int sy
   const size_t smem = fast_smem_bytes(g);
   void (*kern)(const uint16_t*, const uint16_t*, FastGeom, uint16_t*, vwb200_dispi*, ptrdiff_t, uint32_t*, uint16_t*) = nullptr;
   switch (kx) {
-#define KCASE(K) case K: kern = sq ? k1_fast_abs_kernel<K, false, false, true> : (use_float ? k1_fast_abs_kernel<K, true, false> : (float_seed ? k1_fast_abs_kernel<K, false, true> : k1_fast_abs_kernel<K, false, false>)); break;
+#define KCASE(K) case K: kern = sq ? k1_fast_abs_kernel<K, true> : k1_fast_abs_kernel<K, false>; break;
     KCASE(3) KCASE(5) KCASE(7) KCASE(9) KCASE(11) KCASE(13) KCASE(15) KCASE(17) KCASE(19) KCASE(21) KCASE(23) KCASE(25)
     KCASE(27) KCASE(29) KCASE(31)
 #undef KCASE

@@ -29,7 +29,6 @@ struct FastGeom {
   int lox, loy, rox, roy;   // origin of the (logical) left / right rasters inside the images passed to the pack kernels
   int addx, addy;           // constant added to the output disparities
   int sd;                   // k1_screen: dy rows per synchronisation period (ring depth)
-  int dynamic_units;          // k1_screen: 1 = warps draw (octet, half) work units from a shared counter, 0 = static round-robin
 };
 static inline FastGeom make_geom(int W, int H, int sx, int sy, int kx, int ky) {
   FastGeom g;
@@ -42,7 +41,7 @@ static inline FastGeom make_geom(int W, int H, int sx, int sy, int kx, int ky) {
   g.lrows = g.NB * F_TH + ky - 1;
   g.rrows = g.NB * F_TH + ky - 1 + sy;
   g.rw = ((F_COLS + sx + 7) / 8) * 8 + 8;
-  g.lox = g.loy = g.rox = g.roy = 0; g.addx = g.addy = 0; g.scale = F_B; g.dynamic_units = 1; g.sd = 1;
+  g.lox = g.loy = g.rox = g.roy = 0; g.addx = g.addy = 0; g.scale = F_B; g.sd = 1;
   // The work items (strip x band x dy-chunk) are dealt round-robin to 148 persistent CTAs, so the last partial wave idles
   // part of the chip: 1120 items = 7.57 waves run as 8 (efficiency 0.946 -- the 8-GPU share of the 8192^2 raster).  Split
   // the dy range into J chunks (merged by k1_fast_merge) so that items * J fills its last wave: pick the J with the best

@@ -28,8 +28,6 @@
 #include "k1_fast_common.cuh"
 #include <algorithm>
 #include <cmath>
-#include <cstdio>
-#include <cstdlib>
 
 namespace vwb200 {
 
@@ -276,10 +274,6 @@ struct ScreenCtx {           // what the exact evaluation needs
   const float* T0;                          // initial thresholds (lower bound of the cost at a predicted disparity) or null
 };
 
-#ifdef VWB_SCREEN_STATS
-__device__ unsigned long long g_screen_stats[8];   // candidates, warp events, survivors, overflow, flushes
-#endif
-
 // shared-memory accesses by 32-bit shared-window address (no generic-pointer arithmetic on the rare path)
 __device__ __forceinline__ float lds_volatile_f32(uint32_t a) {
   float v;
@@ -302,9 +296,6 @@ struct CandCtx { uint4* list; unsigned char* nan_band; int cap; int W; int cnt; 
 // index inside the chunk); t_sa = shared address of the pixel's threshold, c_sa = shared address of the CandCtx.
 template <int MODE>
 __device__ __noinline__ void screen_candidate(uint32_t t_sa, uint32_t c_sa, uint32_t key, int sprime, float f, float A, float nB, float Qi) {
-#ifdef VWB_SCREEN_STATS
-  atomicAdd(&g_screen_stats[0], 1ull);
-#endif
   const float T = lds_volatile_f32(t_sa);
   if (!(T < INFINITY)) return;                          // pixel closed (outside the raster, or marked for replay)
   const CandCtx* cc = reinterpret_cast<const CandCtx*>(__cvta_shared_to_generic(c_sa));
@@ -332,9 +323,6 @@ __device__ __noinline__ void screen_candidate(uint32_t t_sa, uint32_t c_sa, uint
   else {                                                // list full: replay the pixel instead
     cc->nan_band[(size_t)(pix >> 8) * cc->W + (pix & 255)] = 1;
     atoms_max_s32(t_sa, 0x7f800000);
-#ifdef VWB_SCREEN_STATS
-    atomicAdd(&g_screen_stats[3], 1ull);
-#endif
   }
 }
 
@@ -439,9 +427,6 @@ __device__ __forceinline__ void screen_pass(const int16_t* __restrict__ ltile, c
       for (int b = 0; b < F_B; ++b) {
         if (!FULL && b >= nb) break;
         if (!__any_sync(0xffffffffu, (hit >> b) & 1u)) continue;
-#ifdef VWB_SCREEN_STATS
-        if (lane == 0) atomicAdd(&g_screen_stats[1], 1ull);
-#endif
         int p[8], o[8];
         p[0] = V[0][b];
 #pragma unroll
@@ -501,9 +486,6 @@ __device__ __forceinline__ void screen_flush(const ScreenCtx& cx, const float* _
         const unsigned long long old = atomicMax(bk + pix, key);
         if (key > old) bi[pix] = 0x7fffffff;
         v.z = (uint32_t)key; v.w = (uint32_t)(key >> 32);
-#ifdef VWB_SCREEN_STATS
-        atomicAdd(&g_screen_stats[2], 1ull);
-#endif
       }
     }
     if (!alive) v.x = 0xffffffffu;
@@ -536,7 +518,7 @@ k1_screen_kernel(const int16_t* __restrict__ L16, const int16_t* __restrict__ R1
   uint64_t* bars = reinterpret_cast<uint64_t*>(aring + (size_t)(MODE == M_NCC ? 2 : 1) * NQ_SLOTS * G.rw);
   CandCtx* cc = reinterpret_cast<CandCtx*>(bars + 2);
   const uint32_t c_sa = smem_u32(cc);
-  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  const int tid = threadIdx.x, lane = tid & 31;
   const int ngroups = (G.sx + F_B - 1) / F_B, nunits = ngroups * F_HALVES;
   unsigned long long* bk = bk_all + (size_t)blockIdx.x * F_TH * F_COLS;
   int* bi = bi_all + (size_t)blockIdx.x * F_TH * F_COLS;
@@ -600,15 +582,10 @@ k1_screen_kernel(const int16_t* __restrict__ L16, const int16_t* __restrict__ R1
       }
       // work units of this period = (dy, dx octet, row half); warps draw them from a shared counter: unit durations
       // differ (candidate handling around the cost peak), a static split leaves warps waiting at the barrier
-      for (int uu = 0;; ++uu) {
-        int u;
-        if (G.dynamic_units) {
-          u = 0;
-          if (lane == 0) u = atoms_add_s32(c_sa + (uint32_t)offsetof(CandCtx, next) + 4u * (per & 1), 1);
-          u = __shfl_sync(0xffffffffu, u, 0);
-        } else {
-          u = w + F_WARPS * uu;                            // static round-robin: unit u -> (octet u % ngroups, half u / ngroups)
-        }
+      for (;;) {
+        int u = 0;
+        if (lane == 0) u = atoms_add_s32(c_sa + (uint32_t)offsetof(CandCtx, next) + 4u * (per & 1), 1);
+        u = __shfl_sync(0xffffffffu, u, 0);
         if (u >= nunits * dcur) break;
         const int dy = dyp + u / nunits, uu2 = u % nunits;
         const int g = uu2 % ngroups, row0 = (uu2 / ngroups) * F_RH;
@@ -628,9 +605,6 @@ k1_screen_kernel(const int16_t* __restrict__ L16, const int16_t* __restrict__ R1
         __syncthreads();
         if (tid == 0) cc->cnt = 0;
         screen_flush<MODE>(cx, thr, list, n, bk, bi, s0, y0, dy0, G.sx, tid);
-#ifdef VWB_SCREEN_STATS
-        if (tid == 0) atomicAdd(&g_screen_stats[4], 1ull);
-#endif
       }
     }
     // ---- results of this band (x chunk) ----
@@ -711,7 +685,6 @@ static int screen_launch_t(ImgF left, ImgF right, int W, int H, int sx, int sy, 
   if (!screen_geom(g, MODE)) { set_error("k1_screen: search width %d does not fit in shared memory", sx); return VWB200_ENOIMPL; }
   g.scale = 1;
   if (org) { g.lox = org->lox; g.loy = org->loy; g.rox = org->rox; g.roy = org->roy; g.addx = org->addx; g.addy = org->addy; }
-  g.dynamic_units = getenv("VWB200_SCREEN_DYNAMIC") ? atoi(getenv("VWB200_SCREEN_DYNAMIC")) : 1;
   int c; double maxc;
   if (!screen_params(MODE, kx, ky, vmin, vmax, &c, &maxc)) { set_error("k1_screen: unsupported value range"); return VWB200_ENOIMPL; }
   const ScreenWs ws = carve(g, MODE, workspace);
@@ -743,8 +716,7 @@ static int screen_launch_t(ImgF left, ImgF right, int W, int H, int sx, int sy, 
   }
   // seeding stage (skipped when the half-resolution problem is outside what k1_fast handles)
   const float* T0 = nullptr;
-  if (!getenv("VWB200_SCREEN_NOSEED") && W >= 64 && H >= 64 &&
-      k1_fast_supported(VWB200_ABSOLUTE_DIFFERENCE, ws.kx2, ws.ky2, ws.sx2, ws.sy2, vmin, vmax, true) == VWB200_OK) {
+  if (W >= 64 && H >= 64 && k1_fast_supported(VWB200_ABSOLUTE_DIFFERENCE, ws.kx2, ws.ky2, ws.sx2, ws.sy2, vmin, vmax, true) == VWB200_OK) {
     const int lw2 = ws.W2 + ws.kx2 - 1, lh2 = ws.H2 + ws.ky2 - 1, rw2 = lw2 + ws.sx2 - 1, rh2 = lh2 + ws.sy2 - 1;
     dim3 b2(32, 8);
     screen_subsample2_kernel<<<dim3((lw2 + 31) / 32, (lh2 + 7) / 8), b2, 0, st>>>(left, g.lox, g.loy, lw2, lh2, ws.L2);
@@ -752,7 +724,7 @@ static int screen_launch_t(ImgF left, ImgF right, int W, int H, int sx, int sy, 
     screen_subsample2_kernel<<<dim3((rw2 + 31) / 32, (rh2 + 7) / 8), b2, 0, st>>>(right, g.rox, g.roy, rw2, rh2, ws.R2);
     VWB_LAUNCH_CHECK();
     VWB_TRY(k1_fast_launch(VWB200_ABSOLUTE_DIFFERENCE, ImgF{ws.L2, lw2, lh2, lw2}, ImgF{ws.R2, rw2, rh2, rw2}, ws.W2, ws.H2, ws.sx2, ws.sy2,
-                           ws.kx2, ws.ky2, vmin, vmax, ws.d2, ws.W2, ws.ws2, ws.ws2_bytes, st));
+                           ws.kx2, ws.ky2, vmin, ws.d2, ws.W2, ws.ws2, ws.ws2_bytes, st));
     screen_seed_kernel<MODE><<<dim3((W + 31) / 32, (H + 7) / 8), b2, 0, st>>>(left, right, ws.d2, ws.W2, g, c, K, ws.Sl, ws.Sr, ws.rp, ws.T0);
     VWB_LAUNCH_CHECK();
     T0 = ws.T0;
@@ -779,17 +751,6 @@ static int screen_launch_t(ImgF left, ImgF right, int W, int H, int sx, int sy, 
   kern<<<grid, F_THREADS, smem, st>>>(ws.L16, ws.R16, ws.Qp, ws.Ap, ws.Bp, g, qrows, cx, ws.bk, ws.bi, ws.list, ws.cap, out, opitch, ws.pk, ws.pi);
   VWB_LAUNCH_CHECK();
   if (ev && ev->e1) cudaEventRecord(ev->e1, st);
-#ifdef VWB_SCREEN_STATS
-  {
-    unsigned long long h[8];
-    cudaStreamSynchronize(st);
-    cudaMemcpyFromSymbol(h, g_screen_stats, sizeof(h));
-    fprintf(stderr, "[screen stats] candidates %llu (%.2f / pixel)  warp events %llu  exact evaluations %llu (%.2f / pixel)  overflow %llu  flushes %llu\n",
-            h[0], (double)h[0] / ((double)W * H), h[1], h[2], (double)h[2] / ((double)W * H), h[3], h[4]);
-    unsigned long long z[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    cudaMemcpyToSymbol(g_screen_stats, z, sizeof(z));
-  }
-#endif
   dim3 b(32, 8), gg((W + 31) / 32, (H + 7) / 8);
   if (g.J > 1) {
     k1_screen_merge_kernel<<<gg, b, 0, st>>>(g, ws.pk, ws.pi, ws.nanflag, out, opitch);

@@ -8,8 +8,8 @@
 //
 // One WARP per tile of a zone (<= 33-K columns x 16 rows), four independent warps per CTA:
 //   * a lane owns two adjacent columns of the K-1 padded tile; lanes 0-15 work on disparity d, lanes 16-31 on d+1
-//   * the tile's left columns live in registers (packed u16 pairs); the right search patch is staged once in shared
-//     memory as u16 (edge clamping applied during the copy)
+//   * the tile's left columns live in registers (packed u16 pairs; WIDE: in shared memory); the right search patch is
+//     staged once in shared memory as u16 (edge clamping applied during the copy)
 //   * per disparity: a running vertical window sum per column (the costs leaving the window come from a register ring,
 //     packed u16 pairs), the horizontal window through 6 lane shuffles per row for the lane's two outputs
 //   * running best per output = min over (cost << ib | d - d_begin): strict '<' in ascending raster order of d, i.e. the
@@ -54,10 +54,11 @@ __device__ __forceinline__ unsigned put_byte(unsigned word, unsigned v, int pos)
   return __byte_perm(word, v, pos == 0 ? 0x3214 : (pos == 1 ? 0x3240 : (pos == 2 ? 0x3410 : 0x4210)));   // pos is a constant after unrolling
 }
 
-// LEAN: the left columns are read from shared memory instead of registers and the wide ring keeps |a-b| (two to a register,
-// squared again when the row leaves the window): ~100 registers instead of 168, four CTAs per SM instead of three.
-template <int COST, int K, bool WIDE, bool LEAN>
-__global__ void __launch_bounds__(ZI_WARPS * 32, LEAN ? 4 : 3)
+// WIDE also reads the left columns from shared memory instead of registers, and its ring keeps |a-b| (two to a register,
+// squared again when the row leaves the window): ~100 registers instead of 168, four CTAs per SM instead of three.  The
+// narrow kernel would spill at 128 registers, so it keeps the left columns in registers at three CTAs per SM.
+template <int COST, int K, bool WIDE>
+__global__ void __launch_bounds__(ZI_WARPS * 32, WIDE ? 4 : 3)
 k1_zone_int_kernel(ImgF L, ImgF R, const Zone* __restrict__ zones, const Tile* __restrict__ tiles, int ntiles, float vmin, int ib,
                    int warp_u16, vwb200_dispi* __restrict__ out, double* __restrict__ scratch_cost, int* __restrict__ scratch_idx,
                    int* __restrict__ zone_flag) {
@@ -66,8 +67,8 @@ k1_zone_int_kernel(ImgF L, ImgF R, const Zone* __restrict__ zones, const Tile* _
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, half = lane >> 4, hl = lane & 15;
   const int ti = blockIdx.x * ZI_WARPS + warp;
   if (ti >= ntiles) return;                                    // warps are independent: no CTA-wide barrier below
-  unsigned* sL = reinterpret_cast<unsigned*>(zi_smem + (size_t)warp * warp_u16);     // LEAN: [PH][16] column pairs of the left tile
-  unsigned short* sR = zi_smem + (size_t)warp * warp_u16 + (LEAN ? PH * 32 : 0);
+  unsigned* sL = reinterpret_cast<unsigned*>(zi_smem + (size_t)warp * warp_u16);     // WIDE: [PH][16] column pairs of the left tile
+  unsigned short* sR = zi_smem + (size_t)warp * warp_u16 + (WIDE ? PH * 32 : 0);
   const Tile t = tiles[ti];
   const Zone z = zones[t.zone];
   const int ntx = (z.w + TW - 1) / TW, twb = (z.w + ntx - 1) / ntx;           // balanced split of the zone (host: same formula)
@@ -81,7 +82,7 @@ k1_zone_int_kernel(ImgF L, ImgF R, const Zone* __restrict__ zones, const Tile* _
   const int rph = ph + dy_hi - dy_lo, rpitch = 32 + z.sx;
   const int lx0 = z.lx + t.tx, ly0 = z.ly + t.ty, rx0 = z.rx + t.tx, ry0 = z.ry + t.ty;
 
-  unsigned Lp[LEAN ? 1 : PH];                                  // the lane's two left columns, all padded rows
+  unsigned Lp[WIDE ? 1 : PH];                                  // the lane's two left columns, all padded rows
   bool frac = false;                                           // a non-integer pixel (the mean that replaced a masked one)
 #pragma unroll
   for (int r = 0; r < PH; ++r) {
@@ -89,7 +90,7 @@ k1_zone_int_kernel(ImgF L, ImgF R, const Zone* __restrict__ zones, const Tile* _
     const float f0 = zi_ld(L, lx0 + 2 * hl, ly0 + rr), f1 = zi_ld(L, lx0 + 2 * hl + 1, ly0 + rr);
     frac |= f0 != rintf(f0) || f1 != rintf(f1);
     const unsigned pr = (unsigned)(int)(f0 - vmin) | ((unsigned)(int)(f1 - vmin) << 16);
-    if (LEAN) { if (!half) sL[r * 16 + hl] = pr; } else Lp[r] = pr;
+    if (WIDE) { if (!half) sL[r * 16 + hl] = pr; } else Lp[r] = pr;
   }
   for (int r = 0; r < rph; ++r) {
     const int gy = ry0 + dy_lo + r;
@@ -122,16 +123,15 @@ k1_zone_int_kernel(ImgF L, ImgF R, const Zone* __restrict__ zones, const Tile* _
     const unsigned short* rp = sR + (dy - dy_lo) * rpitch + 2 * hl + dx;
     const unsigned didx = (unsigned)(d - d_begin);
     unsigned v0 = 0, v1 = 0;
-    unsigned ring[WIDE && !LEAN ? 2 * ZI_TH : ZI_TH];          // costs that will leave the window: rows 0 .. TH-1 only
+    unsigned ring[ZI_TH];                                      // costs that will leave the window: rows 0 .. TH-1 only
 #pragma unroll
     for (int r = 0; r < K - 1; ++r) {                          // rows above the first window (ph >= K: always present)
-      const unsigned lp = LEAN ? sL[r * 16 + hl] : Lp[r];
+      const unsigned lp = WIDE ? sL[r * 16 + hl] : Lp[r];
       const int e0 = (int)(lp & 0xffffu) - (int)rp[r * rpitch], e1 = (int)(lp >> 16) - (int)rp[r * rpitch + 1];
       const unsigned c0 = (unsigned)(COST == VWB200_SQUARED_DIFFERENCE ? e0 * e0 : abs(e0));
       const unsigned c1 = (unsigned)(COST == VWB200_SQUARED_DIFFERENCE ? e1 * e1 : abs(e1));
       if (r < ZI_TH) {
-        if (WIDE && LEAN) ring[r] = (unsigned)abs(e0) | ((unsigned)abs(e1) << 16);
-        else if (WIDE) { ring[2 * r] = c0; ring[2 * r + 1] = c1; }
+        if (WIDE) ring[r] = (unsigned)abs(e0) | ((unsigned)abs(e1) << 16);
         else ring[r] = c0 | (c1 << 16);
       }
       v0 += c0; v1 += c1;
@@ -142,13 +142,12 @@ k1_zone_int_kernel(ImgF L, ImgF R, const Zone* __restrict__ zones, const Tile* _
 #pragma unroll                                                 // interleave; rows past th inside the last block work on stale data
         for (int y = yb; y < yb + ZI_RB; ++y) {                // (shared memory rows that exist, outputs never written)
           const int r = y + K - 1;
-          const unsigned lp = LEAN ? sL[r * 16 + hl] : Lp[r];
+          const unsigned lp = WIDE ? sL[r * 16 + hl] : Lp[r];
           const int e0 = (int)(lp & 0xffffu) - (int)rp[r * rpitch], e1 = (int)(lp >> 16) - (int)rp[r * rpitch + 1];
           const unsigned c0 = (unsigned)(COST == VWB200_SQUARED_DIFFERENCE ? e0 * e0 : abs(e0));
           const unsigned c1 = (unsigned)(COST == VWB200_SQUARED_DIFFERENCE ? e1 * e1 : abs(e1));
           if (r < ZI_TH) {
-            if (WIDE && LEAN) ring[r] = (unsigned)abs(e0) | ((unsigned)abs(e1) << 16);
-            else if (WIDE) { ring[2 * r] = c0; ring[2 * r + 1] = c1; }
+            if (WIDE) ring[r] = (unsigned)abs(e0) | ((unsigned)abs(e1) << 16);
             else ring[r] = c0 | (c1 << 16);
           }
           v0 += c0; v1 += c1;
@@ -163,14 +162,9 @@ k1_zone_int_kernel(ImgF L, ImgF R, const Zone* __restrict__ zones, const Tile* _
             if (h1 < bmin[y][1]) bidx[y / 2] = put_byte(bidx[y / 2], didx, (2 * y + 1) & 3);
             bmin[y][0] = min(bmin[y][0], h0);
             bmin[y][1] = min(bmin[y][1], h1);
-            if (LEAN) {
-              const unsigned a0 = ring[y] & 0xffffu, a1 = ring[y] >> 16;
-              v0 -= a0 * a0;
-              v1 -= a1 * a1;
-            } else {
-              v0 -= ring[2 * y];
-              v1 -= ring[2 * y + 1];
-            }
+            const unsigned a0 = ring[y] & 0xffffu, a1 = ring[y] >> 16;
+            v0 -= a0 * a0;
+            v1 -= a1 * a1;
           } else {
             bmin[y][0] = min(bmin[y][0], (h0 << ib) | didx);
             bmin[y][1] = min(bmin[y][1], (h1 << ib) | didx);
@@ -246,18 +240,12 @@ int k1_zone_int_mode(int cost, int kx, int ky, long long range, int* ib_out) {
   return 0;
 }
 bool k1_zone_int_supported(int cost, int kx, int ky, long long range, int* ib_out) { return k1_zone_int_mode(cost, kx, ky, range, ib_out) != 0; }
-// LEAN is the default of the wide variant (+5 % on config 3: 16 instead of 12 warps per SM); the narrow one spills at 128
-// registers and stays fat.  VWB200_ZONE_LEAN / VWB200_ZONE_FAT force either for experiments.
-static bool zi_lean(int mode) {
-  static const int force = getenv("VWB200_ZONE_LEAN") ? 1 : (getenv("VWB200_ZONE_FAT") ? -1 : 0);
-  return force ? force > 0 : mode == 2;
-}
 int k1_zone_int_tile_w(int k) { return 33 - k; }
 int k1_zone_int_tile_h() { return ZI_TH; }
 // u16 elements of right search patch one warp stages for a tile of this zone (upper bound over its tiles)
 long long k1_zone_int_stage_u16(int k, int sx, int sy, int nchunks, int ib) {
   const int span = nchunks > 1 ? std::min(sy, ((1 << ib) + sx - 1) / sx + 1) : sy;
-  return (long long)(ZI_TH + k - 1 + span - 1) * (32 + sx) + (ZI_TH + k - 1) * 32;      // + the left tile (LEAN)
+  return (long long)(ZI_TH + k - 1 + span - 1) * (32 + sx) + (ZI_TH + k - 1) * 32;      // + the left tile (wide)
 }
 long long k1_zone_int_stage_max() { return ZI_MAX_U16; }
 
@@ -271,12 +259,9 @@ int k1_zone_int_launch(int cost, ImgF left, ImgF right, const Zone* d_zones, con
   void (*kern)(ImgF, ImgF, const Zone*, const Tile*, int, float, int, int, vwb200_dispi*, double*, int*, int*) = nullptr;
 #define ZI_CASE(KK)                                                                                                          \
   case KK:                                                                                                                   \
-    if (zi_lean(mode)) kern = mode == 2 ? k1_zone_int_kernel<VWB200_SQUARED_DIFFERENCE, KK, true, true>                          \
-                : (cost == VWB200_SQUARED_DIFFERENCE ? k1_zone_int_kernel<VWB200_SQUARED_DIFFERENCE, KK, false, true>        \
-                                                     : k1_zone_int_kernel<VWB200_ABSOLUTE_DIFFERENCE, KK, false, true>);     \
-    else kern = mode == 2 ? k1_zone_int_kernel<VWB200_SQUARED_DIFFERENCE, KK, true, false>                                   \
-                : (cost == VWB200_SQUARED_DIFFERENCE ? k1_zone_int_kernel<VWB200_SQUARED_DIFFERENCE, KK, false, false>       \
-                                                     : k1_zone_int_kernel<VWB200_ABSOLUTE_DIFFERENCE, KK, false, false>);    \
+    kern = mode == 2 ? k1_zone_int_kernel<VWB200_SQUARED_DIFFERENCE, KK, true>                                               \
+         : (cost == VWB200_SQUARED_DIFFERENCE ? k1_zone_int_kernel<VWB200_SQUARED_DIFFERENCE, KK, false>                     \
+                                              : k1_zone_int_kernel<VWB200_ABSOLUTE_DIFFERENCE, KK, false>);                  \
     break;
   switch (k) {
     ZI_CASE(3) ZI_CASE(5) ZI_CASE(7) ZI_CASE(9) ZI_CASE(11) ZI_CASE(13) ZI_CASE(15) ZI_CASE(17) ZI_CASE(19) ZI_CASE(21) ZI_CASE(23) ZI_CASE(25)

@@ -295,9 +295,9 @@ __global__ void __launch_bounds__(256) sgm_meta_kernel(const short4* __restrict_
 // ---- Hamming costs (get_hamming_distance_costs, SGM.cc:39-73) ---------------------------------------------------------
 // one warp per 32 consecutive pixels: lane i fetches record i (coalesced), then the warp walks the 32 pixels with
 // lanes = the pixel's disparities (coalesced byte stores into the ragged volume); 4 pixels in flight per iteration
-// only_big != 0: the warps whose 32 pixels all have <= 32 entries were done by sgm_cost_lanes_kernel
+// warps whose 32 pixels all have <= 32 entries are skipped: sgm_cost_lanes_kernel does those
 __global__ void __launch_bounds__(256) sgm_cost_kernel(const unsigned long long* __restrict__ lc, const unsigned long long* __restrict__ rc,
-                                                       const SgmMeta* __restrict__ meta, SgmGeom g, sgm_cost_t* __restrict__ cost, int only_big) {
+                                                       const SgmMeta* __restrict__ meta, SgmGeom g, sgm_cost_t* __restrict__ cost) {
   const int lane = threadIdx.x & 31;
   const size_t npix = (size_t)g.ow * g.oh;
   const size_t p0 = (((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * 32;
@@ -307,7 +307,7 @@ __global__ void __launch_bounds__(256) sgm_cost_kernel(const unsigned long long*
   unsigned long long l = 0;
   int br = 0, bc = 0;
   if (mine < npix) mq = __ldg(reinterpret_cast<const uint4*>(meta) + mine);
-  if (only_big && !__any_sync(0xffffffffu, (mq.w >> 8) > 32u)) return;
+  if (!__any_sync(0xffffffffu, (mq.w >> 8) > 32u)) return;
   if (mine < npix) {
     const int c = (int)(mine % g.ow), r = (int)(mine / g.ow);
     br = r + g.min_row - g.hk; bc = c + g.min_col - g.hk;
@@ -355,7 +355,7 @@ __global__ void __launch_bounds__(256) sgm_cost_lanes_kernel(const unsigned long
   uint4 mq = make_uint4(0xffff0000u, 0xffffu, 0u, 0u);
   if (mine < npix) mq = __ldg(reinterpret_cast<const uint4*>(meta) + mine);
   const unsigned n = mine < npix ? (mq.w >> 8) : 0u;
-  if (__any_sync(0xffffffffu, n > 32u)) return;                          // sgm_cost_kernel(only_big) takes this warp
+  if (__any_sync(0xffffffffu, n > 32u)) return;                          // sgm_cost_kernel takes this warp
   const unsigned st0 = __shfl_sync(0xffffffffu, mq.z, 0);                 // pixel p0 always exists
   unsigned end = n ? mq.z + n : st0;
   for (int o = 16; o > 0; o >>= 1) end = max(end, __shfl_xor_sync(0xffffffffu, end, o));
@@ -793,28 +793,25 @@ int sgm_run(const SgmArgs& a, Arena& /*callers_arena*/, cudaStream_t st) {
   VWB_CUDA(cudaMemsetAsync(accum, 0, 64 * sizeof(sgm_accum_t), st));
   cost += 64; accum += 64;
   parts[0] = accum;
-  const int naccum = (a.use_mgm || getenv("VWB200_SGM_SERIAL")) ? 1 : 4;       // partial volumes of the concurrent directions
+  const int naccum = a.use_mgm ? 1 : 4;       // partial volumes of the concurrent SGM directions; MGM sums into accum
   for (int k = 1; k < naccum; ++k) {
     VWB_TRY(ar.alloc(&parts[k], (size_t)total + 192));
     VWB_CUDA(cudaMemsetAsync(parts[k], 0, 64 * sizeof(sgm_accum_t), st));
     parts[k] += 64;
   }
   static_assert(sizeof(sgm_cost_t) == 1, "the staged copy moves bytes");
-  const int lanes_path = getenv("VWB200_SGM_COST_OLD") ? 0 : 1;
-  if (lanes_path) {
-    sgm_cost_lanes_kernel<<<(unsigned)((npix + 255) / 256), 256, 0, st>>>(lc, rc, meta, g, cost);
-    VWB_LAUNCH_CHECK();
-  }
-  sgm_cost_kernel<<<(unsigned)((npix + 255) / 256), 256, 0, st>>>(lc, rc, meta, g, cost, lanes_path);
+  sgm_cost_lanes_kernel<<<(unsigned)((npix + 255) / 256), 256, 0, st>>>(lc, rc, meta, g, cost);
+  VWB_LAUNCH_CHECK();
+  sgm_cost_kernel<<<(unsigned)((npix + 255) / 256), 256, 0, st>>>(lc, rc, meta, g, cost);
   VWB_LAUNCH_CHECK();
   VWB_CUDA(cudaStreamSynchronize(st));                                  // max_n
   if (a.use_mgm) {
     VWB_CUDA(cudaMemsetAsync(accum, 0, ((size_t)total + 64) * sizeof(sgm_accum_t), st));
     VWB_TRY(mgm_paths_launch(meta, cost, accum, l8, g, (size_t)total, ar, st));
   } else {
-    VWB_TRY(sgm_paths_launch(meta, cost, parts, naccum, g, maxes[0], maxes[1], maxes[2], ar, st));
+    VWB_TRY(sgm_paths_launch(meta, cost, parts, g, maxes[0], maxes[1], maxes[2], ar, st));
   }
-  const bool fused_wta = naccum == 4 && maxes[0] <= 32 && !getenv("VWB200_SGM_WTA_UNFUSED");   // every pixel has <= 32 entries
+  const bool fused_wta = naccum == 4 && maxes[0] <= 32;   // every pixel has <= 32 entries
   if (naccum == 4 && !fused_wta) {
     const size_t nvec = ((size_t)total + 7) / 8;              // the volumes are 16-byte aligned and padded
     sgm_sum4_kernel<<<148 * 8, 256, 0, st>>>(reinterpret_cast<uint4*>(accum), reinterpret_cast<const uint4*>(parts[1]),

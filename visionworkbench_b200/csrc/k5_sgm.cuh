@@ -60,7 +60,7 @@ int sgm_run(const SgmArgs& a, Arena& ar, cudaStream_t st);
 int sgm_bounds_run(const SgmArgs& a, int ow, int oh, int* d_bounds, Arena& ar, cudaStream_t st);
 
 // k5_sgm_paths.cu
-int sgm_paths_launch(const SgmMeta* meta, const sgm_cost_t* cost, sgm_accum_t* const* accum, int naccum, const SgmGeom& g, unsigned max_n,
+int sgm_paths_launch(const SgmMeta* meta, const sgm_cost_t* cost, sgm_accum_t* const* accum, const SgmGeom& g, unsigned max_n,
                      unsigned max_w, unsigned max_h, Arena& ar, cudaStream_t st);
 int mgm_paths_launch(const SgmMeta* meta, const sgm_cost_t* cost, sgm_accum_t* accum, const uint8_t* left8, const SgmGeom& g,
                      size_t total, Arena& ar, cudaStream_t st);

@@ -503,7 +503,7 @@ static int sgm_direction_launch(bool rows, const SgmMeta* meta, const sgm_cost_t
 // are independent: they run FOUR AT A TIME on four streams, each pair of directions into its own partial volume
 // (accum[k] receives directions k and k + 4; the first one stores without reading), and the winner-takes-all kernel sums
 // the four partial volumes on the fly.
-int sgm_paths_launch(const SgmMeta* meta, const sgm_cost_t* cost, sgm_accum_t* const* accum, int naccum, const SgmGeom& g, unsigned max_n,
+int sgm_paths_launch(const SgmMeta* meta, const sgm_cost_t* cost, sgm_accum_t* const* accum, const SgmGeom& g, unsigned max_n,
                      unsigned max_w, unsigned max_h, Arena& ar, cudaStream_t st) {
   static const int DIRS[8][2] = {{1, 0}, {0, 1}, {1, 1}, {-1, 1}, {-1, 0}, {0, -1}, {1, -1}, {-1, -1}};
   const bool rows = max_w <= 6 && max_h <= 8 && !getenv("VWB200_SGM_LANES_PER_ENTRY");
@@ -512,11 +512,7 @@ int sgm_paths_launch(const SgmMeta* meta, const sgm_cost_t* cost, sgm_accum_t* c
   unsigned per_warp = 0;
   if (!rows && max_n > 32) {
     per_warp = 2 * ((max_n + 31u) & ~31u);
-    for (int k = 0; k < naccum; ++k) VWB_TRY(ar.alloc(&scratch[k], (size_t)per_warp * nlines));
-  }
-  if (naccum == 1) {
-    for (int i = 0; i < 8; ++i) VWB_TRY(sgm_direction_launch(rows, meta, cost, accum[0], g, DIRS[i][0], DIRS[i][1], i == 0, scratch[0], per_warp, st));
-    return VWB200_OK;
+    for (int k = 0; k < 4; ++k) VWB_TRY(ar.alloc(&scratch[k], (size_t)per_warp * nlines));
   }
   struct Side { cudaStream_t s = nullptr; cudaEvent_t e = nullptr; ~Side() { if (e) cudaEventDestroy(e); if (s) cudaStreamDestroy(s); } } side[3];
   cudaEvent_t fork;
